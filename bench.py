@@ -2,6 +2,7 @@
 """bench.py -- training throughput of the RNN hot path in user-sequences/sec.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c1|c2|c3|c4|c5]
+                    [--dump-outputs DIR]
 
 A "step" is one call of the reference's `train_function(*batch)` (neural_networks/rnn_base.py:290):
 gather -> recurrent scan -> output projection + loss -> BPTT -> scatter -> (all-reduce) -> Adam, on one
@@ -28,8 +29,24 @@ One JSON line on stdout (rank 0):
   multi_rank_cost_check  (N > 1, C1/C2) the all-reduced global cost of step 0 against a one-rank replay of the same
              global batch; parity / parity_max_abs (N = 1) the step-0 cost against the CPU port.
 
+The device-timed region holds exactly K = --steps steps.  Without --steps, K is the config's `steps`, chosen for about
+1 s of device time on one B200 (C2: 2000 steps, 1.30 s on a B200 at its 1000 W power limit and 1965 MHz), so the
+window is long enough to average out the clock and the scheduler and for the clock sampler to see the load.  The K
+steps cycle over min(K, MAX_BATCHES) distinct batches (timed step i uses batch W + i % that), so a large K needs no
+more host-built batches or HBM slots.  Before the timed region run W warm-up steps and one untimed pass over those
+batches, so the number of steps before the last timed one depends only on the arguments.
+
+`--dump-outputs DIR` (e.g. bench_outputs/<build>, which git ignores) then writes what the last timed step computed --
+its cost and the parameters it left, as a caller of train_function sees them -- to DIR/*.npy (see dump_outputs).  The
+inputs are seeded, so the dumps of two builds compare output for output.  The library sums gradients with
+floating-point atomics, and Adam turns the rounding differences of near-zero gradients into full-size steps, so
+trajectories drift apart with the step count: two runs of one build on C2 agree to 1e-5 after W=5 and K=20, but not
+after the default K=2000 (median parameter difference 0.05).  Compare builds on a short run such as --steps 20.
+
 `--impl reference` times that CPU restatement alone (the reference itself -- Python 2 + Theano +
-Lasagne -- cannot be installed here; see DESIGN.md) with all host threads numpy's BLAS will use.
+Lasagne -- cannot be installed here; see DESIGN.md) with all host threads numpy's BLAS will use.  It runs every one
+of its K steps (default REFERENCE_STEPS) with no time limit; on an 8-core Xeon host a step took 1.7 s for C2 (128
+rows), 6.9 s for C4 and 12.2 s for C5 (16 rows each, gradients only), plus the synthetic data set on first use.
 """
 import argparse
 import json
@@ -47,27 +64,37 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 CONFIGS = {
-    # name: model + data shape; B = rows per GPU (weak scaling), gpus = the GPU count BASELINE.json quotes the config on
+    # name: model + data shape; B = rows per GPU (weak scaling), gpus = the GPU count BASELINE.json quotes it on;
+    # steps = the default --steps of the B200 arm, about 1 s of device time on one B200 (ms/step in profiles/README.md;
+    # C1 0.125 ms/step measured)
     "c1": dict(label="C1 RNNOneHot GRU-1x100, 500 items, 200 users, seq-len<=20, batch 16",
                model="onehot", loss="CCE", cell="GRU", layers=(100,), n_items=500, n_users=200, T=20, B=16,
-               uniform_len=(5, 40), gpus=1),
+               uniform_len=(5, 40), gpus=1, steps=8000),
     "c2": dict(label="C2 RNNOneHot LSTM-1x200, ML-1M shape (3706 items, 6040 users, mean len 165), max_length 200, "
                      "batch 128/GPU, full softmax + CCE, Adam",
                model="onehot", loss="CCE", cell="LSTM", layers=(200,), n_items=3706, n_users=6040, T=200, B=128,
-               uniform_len=None, gpus=1),
+               uniform_len=None, gpus=1, steps=2000),
     "c3": dict(label="C3 RNNSampling BPR (S=32; 'BPR-max' does not exist in the reference) LSTM-2x256, 50k items, "
                      "max_length 200, batch 512/GPU, Adam",
                model="sampling", loss="BPR", S=32, cell="LSTM", layers=(256, 256), n_items=50000, n_users=6040, T=200,
-               B=512, uniform_len=None, gpus=1),
+               B=512, uniform_len=None, gpus=1, steps=120),
     "c4": dict(label="C4 RNNMargin hinge over the full catalog (the reference has no sampled-target margin) "
                      "LSTM-1x512, 200k items, max_length 200, batch 1024 over 4 GPUs = 256/GPU, Adam",
                model="margin", loss="hinge", cell="LSTM", layers=(512,), n_items=200000, n_users=6040, T=200, B=256,
-               uniform_len=None, gpus=4),
+               uniform_len=None, gpus=4, steps=120),
     "c5": dict(label="C5 RNNOneHot GRU-2x512, 500k items, max_length 500, batch 2048 over 8 GPUs = 256/GPU, full "
                      "softmax + CCE, Adam",
                model="onehot", loss="CCE", cell="GRU", layers=(512, 512), n_items=500000, n_users=6040, T=500, B=256,
-               uniform_len=None, gpus=8),
+               uniform_len=None, gpus=8, steps=60),
 }
+MAX_BATCHES = 128     # distinct batches the timed steps cycle over: timed step i uses batch W + i % min(K, MAX_BATCHES)
+REFERENCE_STEPS = 5   # default --steps of the reference arm (seconds per step on the host, see the docstring)
+
+
+def timed_batches(W, K):
+    """Batch indices of the K timed steps."""
+    nb = min(K, MAX_BATCHES)
+    return [W + i % nb for i in range(K)]
 
 
 def log(*a):
@@ -135,6 +162,27 @@ def make_batches(predictor, dataset, n):
     finally:
         sys.stdout = stdout
         devnull.close()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, cost, names, params):
+    """cost.npy (float64 [1]) and one float32 param_<ii>_<name>.npy per parameter, at most DUMP_LIMIT_BYTES in all.
+    When the parameters do not fit, each one larger than an equal share of the limit is replaced by a sample of its
+    flattened entries at indices drawn from RandomState(<ii>) (file name ending in .sample), the same in every run."""
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "cost.npy"), np.array([cost], np.float64))
+    room = (DUMP_LIMIT_BYTES - 4096 * (len(params) + 1)) // 4      # float32 entries; 4 KB per file for its header
+    share = room // len(params)
+    sample = sum(p.size for p in params) > room
+    for i, (name, p) in enumerate(zip(names, params)):
+        fname = "param_%02d_%s" % (i, name)
+        a = np.asarray(p, np.float32)
+        if sample and a.size > share:
+            idx = np.sort(np.random.RandomState(i).randint(0, a.size, share))
+            a, fname = a.reshape(-1)[idx], fname + ".sample"
+        np.save(os.path.join(dirname, fname + ".npy"), a)
 
 
 def n_out_columns(cfg, B_global):
@@ -282,20 +330,24 @@ class ClockSampler(object):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=60)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: the config's 'steps' for the B200 arm, %d for the reference arm)"
+                         % REFERENCE_STEPS)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--rows-per-gpu", type=int, default=0, help="override the per-GPU batch of the config")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--min-timed-s", type=float, default=1.2,
-                    help="the K timed steps are repeated back to back until the timed region is at least this long")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the cost and the parameters left by the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 path computed; it needs --impl b200")
     cfg = dict(CONFIGS[args.config])
     if args.rows_per_gpu > 0:
         cfg["B"] = args.rows_per_gpu
     W = max(args.warmup, 3) if args.impl == "b200" else args.warmup
-    K = args.steps
+    K = args.steps if args.steps is not None else (cfg["steps"] if args.impl == "b200" else REFERENCE_STEPS)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -314,7 +366,7 @@ def main():
             "config": {"workload": cfg["label"], "global_batch": B_global, "seq_len": cfg["T"],
                        "parallelism": "dp%d" % n_gpus,
                        "l2": "no explicit flush: a step streams more activation bytes than the 126 MB L2 and every "
-                             "step of a repetition uses a different batch"}}
+                             "timed step uses a different batch"}}
 
     # ------------------------------------------------------------------ reference arm (CPU)
     if args.impl == "reference":
@@ -326,7 +378,7 @@ def main():
         # a step = the first `rows` rows of the global mini-batch (bounded sample of the same workload)
         rows = min(B_global, 128 if args.config in ("c1", "c2") else (64 if args.config == "c3" else 16))
         heavy = args.config in ("c4", "c5")      # 0.5-1 G parameters: gradients only, no Adam pass over the arena
-        rate, sec, done, n_rows, _ = cpu_reference_rate(cfg, pred, batches, K, W, rows=rows, budget_s=240.0,
+        rate, sec, done, n_rows, _ = cpu_reference_rate(cfg, pred, batches, K, W, rows=rows, budget_s=float("inf"),
                                                         update=not heavy)
         cores = blas_threads()
         out = dict(base)
@@ -350,7 +402,8 @@ def main():
     nccl_id = ctl.broadcast(_capi.nccl_unique_id() if rank == 0 else None) if ctl else None
 
     dataset = make_dataset(cfg)
-    n_batches = K + W
+    timed = timed_batches(W, K)
+    n_batches = W + min(K, MAX_BATCHES)
     pred = make_predictor(cfg, dataset, n_ranks=n_gpus, rank=rank, nccl_id=nccl_id, device=local_rank,
                           n_slots=n_batches if staged else 1)
     pred._compile_train_function()
@@ -365,9 +418,9 @@ def main():
     def max_over_ranks(x):
         return ctl.all_max(x) if ctl else x
 
-    def run_steps(lo, hi, want_cost=False):
+    def run_steps(idx, want_cost=False):
         c = None
-        for i in range(lo, hi):
+        for i in idx:
             if staged:
                 c = eng.train_step_staged(i, want_cost=want_cost)
             else:
@@ -383,33 +436,31 @@ def main():
     step0_cost = None
     if staged:
         step0_cost = float(eng.train_step_staged(0, want_cost=True))     # global cost of the first step (parity checks)
-        run_steps(1, W)
+        run_steps(range(1, W))
     else:
         step0_cost = float(pred.train_function(*batches[0]))
-        run_steps(1, W)
+        run_steps(range(1, W))
     eng.synchronize()
-    # estimate a repetition, then repeat the K timed steps until the timed region is long enough for the clock sampler
-    eng.timer_start()
-    t_enq = time.perf_counter()
-    run_steps(W, W + K)
-    host_enqueue_ms = (time.perf_counter() - t_enq) * 1e3 / K     # host time to enqueue a step, launch queue not yet full
-    est_ms = max_over_ranks(eng.timer_stop())
-    R = max(1, int(np.ceil(args.min_timed_s * 1e3 / max(est_ms, 1e-3))))
-    R = int(max_over_ranks(R))
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
         time.sleep(0.15)      # nvidia-smi needs ~0.1 s before its first sample
     barrier()
+    # one untimed pass over the batches of the timed region warms every batch shape it uses; it runs after the
+    # sampler's start-up sleep, so the device is not left idle between the warm pass and the timed steps
+    t_enq = time.perf_counter()
+    run_steps(range(W, n_batches))
+    host_enqueue_ms = (time.perf_counter() - t_enq) * 1e3 / (n_batches - W)     # host enqueue time of a step
     launches0 = eng.kernel_launches()
     eng.timer_start()
-    for _ in range(R):
-        run_steps(W, W + K)
+    run_steps(timed)
     ms = eng.timer_stop()
     barrier()
-    launches = (eng.kernel_launches() - launches0) // R
+    launches = eng.kernel_launches() - launches0
     last_cost = eng.synchronize(want_cost=True)
-    ms = max_over_ranks(ms) / R
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, float(last_cost), [n for n, _ in eng.param_infos()], eng.get_all_param_values())
+    ms = max_over_ranks(ms)
     value = B_global * K / (ms * 1e-3)
 
     # ---- leg 2: end to end through the public API, host buffers ------------------------------
@@ -418,11 +469,10 @@ def main():
     eng.synchronize()
     barrier()
     t0 = time.perf_counter()
-    for _ in range(R):
-        for i in range(W, W + K):
-            cost = pred.train_function(*batches[i])
+    for i in timed:
+        cost = pred.train_function(*batches[i])
     eng.synchronize()
-    e2e_s = max_over_ranks(time.perf_counter() - t0) / R
+    e2e_s = max_over_ranks(time.perf_counter() - t0)
     clocks = sampler.stop() if rank == 0 else None     # sampled across both timed legs
     barrier()
     e2e_value = B_global * K / e2e_s
@@ -435,7 +485,7 @@ def main():
     # ---- leg 3: per-stage device times (separate pass; profiling syncs every step) -------------
     eng.set_profiling(True)
     acc = {}
-    for i in range(W, W + K):
+    for i in timed:
         if staged:
             eng.train_step_staged(i, want_cost=False)
         else:
@@ -443,7 +493,7 @@ def main():
         for k, v in eng.stage_times().items():
             acc[k] = acc.get(k, 0.0) + v / K
     eng.set_profiling(False)
-    works = [step_work(cfg, b, n_gpus) for b in batches[W:W + K]]
+    works = [step_work(cfg, batches[i], n_gpus) for i in timed]
     mean_V = float(np.mean([w["V"] for w in works]))
     peaks = {}
     try:
@@ -496,7 +546,7 @@ def main():
     per_rank = None
     if ctl:
         try:
-            my_valid = float(np.mean([np.asarray(b[1])[rank::n_gpus].sum() for b in batches[W:W + K]]))
+            my_valid = float(np.mean([np.asarray(batches[i][1])[rank::n_gpus].sum() for i in timed]))
         except Exception:
             my_valid = None
         per_rank = ctl.all_gather({"rank": rank, "scan_ms": round(acc.get("rnn_fwd", 0.0) + acc.get("rnn_bwd", 0.0), 4),
@@ -507,7 +557,7 @@ def main():
         out = dict(base)
         if per_rank is not None:
             out["per_rank"] = sorted(per_rank, key=lambda e: e["rank"])
-        out.update({"impl": "b200", "value": value, "ms_per_step": ms / K, "repeats": R, "timed_steps_total": K * R,
+        out.update({"impl": "b200", "value": value, "ms_per_step": ms / K,
                     "host_enqueue_ms_per_step": host_enqueue_ms, "clocks": clocks,
                     "valid_steps_per_s": mean_V * n_gpus * K / (ms * 1e-3),
                     "value_inputs": "device-resident batch slots" if staged else

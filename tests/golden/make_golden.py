@@ -6,11 +6,15 @@ produced by the float64 numpy oracle (oracle/sbr_oracle.py), whose gradients are
 finite differences and by torch.autograd (tests/test_oracle*.py).  PARITY UNPINNED against the real
 reference; regenerate with   python tests/golden/make_golden.py   (deterministic, ~2 s).
 
-Contents: initial parameters (float32, checkpoint order), 8 training batches built by the host mirror
-of RNNBase._gen_mini_batch on a seeded synthetic dataset, the per-step costs of 8 Adam steps
-(float64), the parameters after those steps, and for 20 validation users the input, the goal and the
-oracle's top-10 + recall@10 / sps after training.
+Contents: the initial parameters (float32, checkpoint order) as the seed of oracle.init_params and the
+SHA-256 of their bytes, 8 training batches built by the host mirror of RNNBase._gen_mini_batch on a
+seeded synthetic dataset, the per-step costs of 8 Adam steps (float64), the parameters after those
+steps, and for 20 validation users the input, the goal and the oracle's top-10 + recall@10 / sps after
+training.  Stored whole, the random initial and final parameters would not fit in 1 MB; so each final
+parameter is kept as its step from the initial one, quantised to int16 over the largest step
+(final = init + final_q * final_scale, within final_scale / 2 ~ 1.2e-7 of the float64 oracle).
 """
+import hashlib
 import os
 import random
 import sys
@@ -22,6 +26,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 
 from oracle import sbr_oracle as O  # noqa: E402
+
+
+def init_sha256(vals):
+    return hashlib.sha256(b"".join(np.ascontiguousarray(v, np.float32).tobytes() for v in vals)).hexdigest()
 
 
 def build():
@@ -42,7 +50,8 @@ def build():
     gen = pred._gen_mini_batch(ds.training_set())
     batches = [next(gen) for _ in range(8)]
     spec = O.Spec(n_items=500, cell="GRU", layers=(100,), loss="CCE")
-    init32 = O.init_params(spec, np.random.RandomState(1), np.float32)
+    init_seed = 1
+    init32 = O.init_params(spec, np.random.RandomState(init_seed), np.float32)
     vals = [v.astype(np.float64) for v in init32]
     upd = O.Updater("adam", lr=1e-3)
     costs = []
@@ -66,9 +75,13 @@ def build():
            "val_goal_off": np.cumsum([0] + [len(g) for g in goals]).astype(np.int32),
            "val_seen_flat": np.concatenate([np.asarray(s, np.int32) for s in seen]),
            "val_seen_off": np.cumsum([0] + [len(s) for s in seen]).astype(np.int32)}
+    out["init_seed"] = init_seed
+    out["init_sha256"] = init_sha256(init32)
     for i, (a, b) in enumerate(zip(init32, vals)):
-        out["init_%02d" % i] = a
-        out["final_%02d" % i] = b.astype(np.float32)
+        step = b - a.astype(np.float64)
+        scale = np.abs(step).max() / 32767 or 1.0
+        out["final_q_%02d" % i] = np.round(step / scale).astype(np.int16)
+        out["final_scale_%02d" % i] = scale
     for i, (X, mask, Y, pop, _) in enumerate(batches):
         out["X_%d" % i] = X; out["mask_%d" % i] = mask; out["Y_%d" % i] = Y; out["pop_%d" % i] = pop
     return out
