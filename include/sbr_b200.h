@@ -174,6 +174,35 @@ SBR_API int64_t sbr_kernel_launches(const sbr_model* m);             /* kernels 
  * `lens` may be NULL (static rule).  Touches no device; used by the CPU tests. */
 SBR_API int sbr_plan_scan_tiles(const int32_t* lens, int B, int t_max, int slots, float ratio8,
                                 int* tile_rows, int* n_tiles, int* extra16, unsigned char* order64);
+/* Which recurrent-scan kernel variant one layer (cell, H) runs for a batch of B rows (lengths `lens`, may be NULL) in
+ * one direction, as launch_rnn_forward / launch_rnn_backward decide it.  Families, in the order they are tried: */
+enum { SBR_SCAN_TC_CLUSTER = 0,   /* tcgen05 cluster scans (rnn_tc.cu): <G, BT> forward, <G, MT, BT> backward        */
+       SBR_SCAN_PERSISTENT = 1,   /* persistent tensor-core scans (tc_scan.cu), sliced into co-resident launches     */
+       SBR_SCAN_STEP = 2,         /* one tensor-core kernel per time step (tc_gemm.cu)                               */
+       SBR_SCAN_FFMA = 3 };       /* FFMA cluster scans (rnn_cluster.cu): <G, BT, JU, WSMEM>                         */
+typedef struct sbr_scan_plan {
+  int32_t family;            /* SBR_SCAN_*                                                                         */
+  int32_t G;                 /* gate blocks: 4 LSTM, 3 GRU, 1 Vanilla                                              */
+  int32_t BT;                /* batch rows per tile of the main launch: tcgen05 8|16, FFMA 8|16|32, persistent 128
+                                forward / 32 backward, 0 for the step scans                                        */
+  int32_t MT;                /* tcgen05 backward: 128-unit hidden tiles, else 0                                    */
+  int32_t JU;                /* FFMA: hidden units per lane (1|2), else 0                                          */
+  int32_t wsmem;             /* FFMA: W_hid slice resident in shared memory                                        */
+  int32_t splitk;            /* persistent backward: split-K clusters of 4 CTAs                                    */
+  int32_t C, Hs;             /* hidden-unit ownership: slice r < C holds units [r*Hs, min(H, (r+1)*Hs))            */
+  int32_t launches;          /* scan kernel launches of this layer and direction                                  */
+  int32_t tiles_per_launch;  /* persistent: batch tiles per launch, else 0                                        */
+} sbr_scan_plan;
+/* m != NULL: the handle's switches, SM count and co-resident cluster counts (queried on its device); n_sm, tc_slots
+ * and splitk_slots are ignored.  m == NULL: touches no device; the switches are read from the environment
+ * (SBR_DISABLE_TC, SBR_DISABLE_TC_BWD, SBR_DISABLE_STEP_SCAN, SBR_DISABLE_PERSISTENT_SCAN, SBR_DISABLE_SPLITK_SCAN,
+ * SBR_DISABLE_TC_GEMM, SBR_DISABLE_TMA_GEMM, SBR_TC_BT, ...) and the device is described by n_sm, tc_slots[i] =
+ * co-resident tcgen05 scan clusters of 2^i CTAs (i = 0..3) and splitk_slots = co-resident split-K clusters.
+ * Returns SBR_E_ARG for a layer no scan takes and under SBR_SCAN_MULTICAST.  sbr_scan_launches counts the scan
+ * kernel launches of a handle (part of sbr_kernel_launches). */
+SBR_API int sbr_plan_layer_scan(const sbr_model* m, int cell, int H, int B, const int32_t* lens, int t_max, int backward,
+                                int n_sm, const int32_t* tc_slots, int splitk_slots, sbr_scan_plan* out);
+SBR_API int64_t sbr_scan_launches(const sbr_model* m);
 /* Diagnostics: C[M,N] = alpha * op(A) * op(B) (+ bias[n]) (+ beta * C) on the device the handle lives on, host buffers
  * in and out (row-major; ta: A stored [K,lda]; tb: B stored [N,ldb]; beta in {0,1}; bias may be NULL).  engine 0 = the
  * fp32 FFMA kernels (gemm.cu), 1 = the tcgen05 3xTF32 kernel (tc_gemm.cu), which is what every GEMM-shaped stage of

@@ -47,6 +47,14 @@ class SbrConfig(C.Structure):
     ]
 
 
+class SbrScanPlan(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("family", "G", "BT", "MT", "JU", "wsmem", "splitk", "C", "Hs", "launches",
+                                         "tiles_per_launch")]
+
+
+SCAN_FAMILIES = {0: "tc_cluster", 1: "persistent", 2: "step", 3: "ffma"}
+
+
 _P = C.c_void_p
 _i32p = C.POINTER(C.c_int32)
 _f32p = C.POINTER(C.c_float)
@@ -84,6 +92,9 @@ SIGNATURES = {
     "sbr_kernel_launches": (C.c_int64, [_P]),
     "sbr_plan_scan_tiles": (C.c_int, [_i32p, C.c_int, C.c_int, C.c_int, C.c_float, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                       C.POINTER(C.c_int), C.POINTER(C.c_ubyte)]),
+    "sbr_plan_layer_scan": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _i32p, C.c_int, C.c_int, C.c_int, _i32p, C.c_int,
+                                      C.POINTER(SbrScanPlan)]),
+    "sbr_scan_launches": (C.c_int64, [_P]),
     "sbr_debug_gemm": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _f32p, C.c_int, _f32p, C.c_int,
                                  _f32p, C.c_int, C.c_float, C.c_float, _f32p, C.c_int, _f32p]),
     "sbr_timer_start": (C.c_int, [_P]),
@@ -123,6 +134,35 @@ def _f32(a):
 
 def _ptr(a, typ):
     return a.ctypes.data_as(typ)
+
+
+def _plan_dict(p):
+    d = {n: int(getattr(p, n)) for n, _ in SbrScanPlan._fields_}
+    d["family"] = SCAN_FAMILIES[d["family"]]
+    return d
+
+
+def plan_layer_scan(cell, H, B, backward, lens=None, t_max=None, n_sm=148, tc_slots=(148, 74, 37, 15), splitk_slots=37,
+                    handle=None):
+    """The scan variant the launchers pick for one layer and direction (sbr_plan_layer_scan), as a dict.  Without a
+    handle the device is described by n_sm, tc_slots (co-resident tcgen05 scan clusters of 1, 2, 4, 8 CTAs) and
+    splitk_slots, and the SBR_* switches are read from the environment; returns None when no scan takes the layer."""
+    lib = load_library()
+    lp = None
+    if lens is not None:
+        lens = _i32(lens)
+        lp = _ptr(lens, _i32p)
+    if t_max is None:
+        t_max = int(max(lens)) if lens is not None else 1
+    slots = _i32(tc_slots)
+    out = SbrScanPlan()
+    rc = lib.sbr_plan_layer_scan(handle, CELLS[cell], int(H), int(B), lp, int(t_max), int(bool(backward)), int(n_sm),
+                                 _ptr(slots, _i32p), int(splitk_slots), C.byref(out))
+    if rc == -1:
+        return None
+    if rc != 0:
+        raise SbrError(rc, "sbr_plan_layer_scan")
+    return _plan_dict(out)
 
 
 def nccl_unique_id():
@@ -369,6 +409,13 @@ class Engine(object):
 
     def kernel_launches(self):
         return int(self.lib.sbr_kernel_launches(self._h))
+
+    def scan_launches(self):
+        return int(self.lib.sbr_scan_launches(self._h))
+
+    def plan_layer_scan(self, cell, H, B, backward, lens=None, t_max=None):
+        """The live plan of this handle (its switches, SM count and co-resident cluster counts)."""
+        return plan_layer_scan(cell, H, B, backward, lens, t_max, handle=self._h)
 
     def debug_gemm(self, A, B, ta=False, tb=False, C0=None, alpha=1.0, beta=0.0, bias=None, engine=1, reps=1):
         """op(A) @ op(B) through one of the library's GEMM kernels (diagnostics / tests); returns (C, ms)."""

@@ -108,6 +108,7 @@ struct sbr_model {
   std::string err;
   int err_code = 0;
   int64_t launches = 0;
+  int64_t scan_launches = 0;          // of these, launches of a recurrent-scan kernel (all four families)
 
   // geometry
   int B = 0, T = 0, K = 1, N = 0, n_in = 0, E = 0, L = 0, H_last = 0;
@@ -233,10 +234,26 @@ int launch_rnn_forward(sbr_model* m, const LayerDesc& L, const int32_t* len, int
 int launch_rnn_backward(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max,
                         const float* dh_last /* top layer, else nullptr */);
 
+// Scan dispatch switches of one handle (sbr_create reads them from the environment); sbr_plan_layer_scan without a
+// handle reads the same variables when it is called.
+struct ScanSwitches {
+  bool tc_gemm = true, step = true, persistent = true, tma_gemm = true, splitk = true, multicast = false;
+  bool disable_tc_bwd = false;
+};
+ScanSwitches scan_switches(const sbr_model* m);
+ScanSwitches scan_switches_from_env();
+
 // rnn_tc.cu (returns 1 when the tcgen05 path does not apply)
 int launch_rnn_forward_tc(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, float* h_last);
 int launch_rnn_backward_tc(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, const float* dh_last);
 int tc_scan_applies(int G, int H);   // 1 when both tcgen05 scans handle this layer shape
+// The decisions of the two tcgen05 launchers, for sbr_plan_layer_scan: the cluster shape of a layer (ok = false when
+// tc_plan rejects it; bwd_ok: the backward fits TMEM too), the co-resident clusters of that shape on the current device,
+// and the tile schedule of a batch.
+struct TcShape { bool ok, bwd_ok; int C, Hs, MT; };
+TcShape tc_scan_shape(int G, int H);
+int tc_scan_slots(int G, int H);
+void tc_scan_schedule(const int32_t* hl, int B, int t_max, int slots, bool backward, int* tile_rows, int* n_launches);
 
 // wgrad_tc.cu : dW_hid[H, G*H] += sum_rows h_prev[row]^T da[row] on tcgen05 (3xTF32) from the K-major copies
 int launch_wgrad_stage_list(sbr_model* m, const int32_t* len, int B, int rows);
@@ -247,10 +264,19 @@ int launch_gemm_tc(sbr_model* m, bool ta, bool tb, int M, int N, int K, const fl
                    float* C, int ldc, float alpha, float beta, const float* bias);
 // per-step tensor-core scans for hidden sizes the cluster-resident kernels do not hold
 int step_scan_applies(const sbr_model* m, int G, int H);
+int step_scan_applies(const ScanSwitches& s, int H);
 int launch_rnn_forward_steps(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, float* h_last);
 int launch_rnn_backward_steps(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, const float* dh_last);
 // tc_scan.cu : the same scans as ONE cooperative launch per layer (return 1 when they do not apply)
 int persistent_scan_applies(const sbr_model* m, int G, int H);
+int persistent_scan_applies(const ScanSwitches& s, int H);
+// How the persistent launchers slice a batch: tiles of `tile_rows` rows (128 forward, 32 backward), at most
+// `tiles_per_launch` of them per launch so that every CTA of a launch is co-resident; owner = hidden units per CTA slice
+// (8 forward, 128 backward).  splitk_slots = co-resident 4-CTA split-K clusters (persistent_splitk_slots()).
+struct PersistentSlicing { int tile_rows, n_tiles, tiles_per_launch, owner; bool splitk; };
+PersistentSlicing persistent_fwd_slicing(int n_sm, int H, int B);
+PersistentSlicing persistent_bwd_slicing(int n_sm, int H, int B, bool use_splitk, int splitk_slots);
+int persistent_splitk_slots();
 int launch_rnn_forward_persistent(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, float* h_last);
 int launch_rnn_backward_persistent(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, const float* dh_last);
 

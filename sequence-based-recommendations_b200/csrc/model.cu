@@ -283,6 +283,24 @@ extern "C" void sbr_destroy(sbr_model* m) {
   delete m;
 }
 
+ScanSwitches scan_switches_from_env() {
+  ScanSwitches s;
+  s.tc_gemm = getenv("SBR_DISABLE_TC_GEMM") == nullptr;
+  s.step = getenv("SBR_DISABLE_STEP_SCAN") == nullptr;
+  s.tma_gemm = getenv("SBR_DISABLE_TMA_GEMM") == nullptr;
+  s.persistent = getenv("SBR_DISABLE_PERSISTENT_SCAN") == nullptr;
+  s.splitk = getenv("SBR_DISABLE_SPLITK_SCAN") == nullptr;
+  s.multicast = getenv("SBR_SCAN_MULTICAST") != nullptr;
+  s.disable_tc_bwd = getenv("SBR_DISABLE_TC_BWD") != nullptr;
+  return s;
+}
+ScanSwitches scan_switches(const sbr_model* m) {
+  ScanSwitches s;
+  s.tc_gemm = m->use_tc_gemm; s.step = m->use_step_scan; s.tma_gemm = m->use_tma_gemm; s.persistent = m->use_persistent_scan;
+  s.splitk = m->use_splitk_scan; s.multicast = m->use_scan_multicast; s.disable_tc_bwd = m->disable_tc_bwd;
+  return s;
+}
+
 static int create_impl(sbr_model* m) {
   const sbr_config& c = m->cfg;
   CU_TRY(m, cudaSetDevice(m->dev));
@@ -293,17 +311,18 @@ static int create_impl(sbr_model* m) {
     return SBR_E_NOGPU;
   }
   m->n_sm = prop.multiProcessorCount;
-  m->use_tc_gemm = getenv("SBR_DISABLE_TC_GEMM") == nullptr;
-  m->use_step_scan = getenv("SBR_DISABLE_STEP_SCAN") == nullptr;
-  m->use_tma_gemm = getenv("SBR_DISABLE_TMA_GEMM") == nullptr;
-  m->use_persistent_scan = getenv("SBR_DISABLE_PERSISTENT_SCAN") == nullptr;
+  const ScanSwitches sw = scan_switches_from_env();
+  m->use_tc_gemm = sw.tc_gemm;
+  m->use_step_scan = sw.step;
+  m->use_tma_gemm = sw.tma_gemm;
+  m->use_persistent_scan = sw.persistent;
   if (const char* e = getenv("SBR_SCAN_FENCE")) m->scan_fence_mode = atoi(e);
-  m->use_splitk_scan = getenv("SBR_DISABLE_SPLITK_SCAN") == nullptr;
-  m->use_scan_multicast = getenv("SBR_SCAN_MULTICAST") != nullptr;
+  m->use_splitk_scan = sw.splitk;
+  m->use_scan_multicast = sw.multicast;
   m->no_side_stream = getenv("SBR_NO_SIDE_STREAM") != nullptr;
   m->no_early_cost = getenv("SBR_NO_EARLY_COST") != nullptr;
   m->disable_tc = getenv("SBR_DISABLE_TC") != nullptr;
-  m->disable_tc_bwd = getenv("SBR_DISABLE_TC_BWD") != nullptr;
+  m->disable_tc_bwd = sw.disable_tc_bwd;
   {
     // the critical path (scans) outranks the side stream: when both have CTAs pending, the 8-CTA clusters of a scan
     // must not queue behind the output-layer weight-gradient GEMM
@@ -1249,6 +1268,7 @@ extern "C" int sbr_stage_times(sbr_model* m, float ms[SBR_N_STAGES]) {
 }
 
 extern "C" int64_t sbr_kernel_launches(const sbr_model* m) { return m ? m->launches : SBR_E_ARG; }
+extern "C" int64_t sbr_scan_launches(const sbr_model* m) { return m ? m->scan_launches : SBR_E_ARG; }
 
 extern "C" int sbr_debug_gemm(sbr_model* m, int engine, int ta, int tb, int M, int N, int K, const float* A, int lda,
                               const float* B, int ldb, float* C, int ldc, float alpha, float beta, const float* bias,

@@ -533,7 +533,7 @@ size_t bwd_smem(int G, int BT, int JU, int H, int Hs, int C, bool wsmem) {
 }
 
 // cluster size, batch tile and weight residency for one layer
-Plan make_plan(const sbr_model* m, int G, int H, int B, bool backward) {
+Plan make_plan(int n_sm, int G, int H, int B, bool backward) {
   const size_t limit = 227 * 1024 - 1024;  // static shared memory of the kernels is < 1 KB
   Plan best{};
   int C = 8;
@@ -556,7 +556,7 @@ Plan make_plan(const sbr_model* m, int G, int H, int B, bool backward) {
       const size_t s = backward ? bwd_smem(G, BT, JU, H, Hs, C, wsmem) : fwd_smem(G, BT, JU, H, Hs, wsmem);
       if (s > limit) continue;
       pick = i;
-      if (cdiv(B, BT) * C <= m->n_sm) break;
+      if (cdiv(B, BT) * C <= n_sm) break;
     }
     if (pick >= 0) {
       best.C = C; best.Hs = Hs; best.BT = bts[pick]; best.JU = JU; best.wsmem = wsmem;
@@ -594,22 +594,40 @@ int launch_cluster(sbr_model* m, Kern kern, const Plan& p, int n_tiles, const Rn
     return SBR_E_CUDA;
   }
   m->launches++;
+  m->scan_launches++;
   return 0;
 }
 
+// The FFMA scan variants <G, BT, JU, WSMEM> per direction: exactly the ones make_plan returns for some layer (H <= 512)
+// and batch.  JU = 1 layers (Hs <= 32) always hold their weight slice in shared memory, so no JU = 1 global-weight
+// variant is compiled; tests/test_scan_dispatch.py checks these lists against the planner.
 template <int G, bool BWD>
 int dispatch(sbr_model* m, const Plan& p, int n_tiles, const RnnArgs& a) {
-#define SBR_CASE(BT_, JU_, WS_)                                                              \
-  if (p.BT == BT_ && p.JU == JU_ && p.wsmem == WS_) {                                        \
-    if (BWD) return launch_cluster(m, rnn_bwd_kernel<G, BT_, JU_, WS_>, p, n_tiles, a);      \
-    return launch_cluster(m, rnn_fwd_kernel<G, BT_, JU_, WS_>, p, n_tiles, a);               \
-  }
-  SBR_CASE(8, 1, true) SBR_CASE(16, 1, true) SBR_CASE(32, 1, true)
-  SBR_CASE(8, 2, true) SBR_CASE(16, 2, true)
-  SBR_CASE(8, 1, false) SBR_CASE(16, 1, false) SBR_CASE(32, 1, false)
-  SBR_CASE(8, 2, false) SBR_CASE(16, 2, false)
-#undef SBR_CASE
-  sbr_set_error(m, SBR_E_ARG, "no recurrent kernel for BT=%d JU=%d", p.BT, p.JU);
+#define SBR_FFMA_FWD(G_, BT_, JU_, WS_)                                                      \
+  if constexpr (!BWD && G == G_)                                                             \
+    if (p.BT == BT_ && p.JU == JU_ && p.wsmem == WS_)                                        \
+      return launch_cluster(m, rnn_fwd_kernel<G_, BT_, JU_, WS_>, p, n_tiles, a);
+#define SBR_FFMA_BWD(G_, BT_, JU_, WS_)                                                      \
+  if constexpr (BWD && G == G_)                                                              \
+    if (p.BT == BT_ && p.JU == JU_ && p.wsmem == WS_)                                        \
+      return launch_cluster(m, rnn_bwd_kernel<G_, BT_, JU_, WS_>, p, n_tiles, a);
+  // LSTM: the 16-row JU = 2 forward tile never fits next to a resident weight slice
+  SBR_FFMA_FWD(4, 8, 1, true) SBR_FFMA_FWD(4, 16, 1, true) SBR_FFMA_FWD(4, 32, 1, true)
+  SBR_FFMA_FWD(4, 8, 2, true) SBR_FFMA_FWD(4, 8, 2, false) SBR_FFMA_FWD(4, 16, 2, false)
+  SBR_FFMA_BWD(4, 8, 1, true) SBR_FFMA_BWD(4, 16, 1, true) SBR_FFMA_BWD(4, 32, 1, true)
+  SBR_FFMA_BWD(4, 8, 2, true) SBR_FFMA_BWD(4, 16, 2, true) SBR_FFMA_BWD(4, 8, 2, false) SBR_FFMA_BWD(4, 16, 2, false)
+  SBR_FFMA_FWD(3, 8, 1, true) SBR_FFMA_FWD(3, 16, 1, true) SBR_FFMA_FWD(3, 32, 1, true)
+  SBR_FFMA_FWD(3, 8, 2, true) SBR_FFMA_FWD(3, 16, 2, true) SBR_FFMA_FWD(3, 8, 2, false) SBR_FFMA_FWD(3, 16, 2, false)
+  SBR_FFMA_BWD(3, 8, 1, true) SBR_FFMA_BWD(3, 16, 1, true) SBR_FFMA_BWD(3, 32, 1, true)
+  SBR_FFMA_BWD(3, 8, 2, true) SBR_FFMA_BWD(3, 16, 2, true) SBR_FFMA_BWD(3, 8, 2, false) SBR_FFMA_BWD(3, 16, 2, false)
+  // Vanilla: the weight slice of H <= 512 always fits in shared memory
+  SBR_FFMA_FWD(1, 8, 1, true) SBR_FFMA_FWD(1, 16, 1, true) SBR_FFMA_FWD(1, 32, 1, true)
+  SBR_FFMA_FWD(1, 8, 2, true) SBR_FFMA_FWD(1, 16, 2, true)
+  SBR_FFMA_BWD(1, 8, 1, true) SBR_FFMA_BWD(1, 16, 1, true) SBR_FFMA_BWD(1, 32, 1, true)
+  SBR_FFMA_BWD(1, 8, 2, true) SBR_FFMA_BWD(1, 16, 2, true)
+#undef SBR_FFMA_FWD
+#undef SBR_FFMA_BWD
+  sbr_set_error(m, SBR_E_ARG, "no recurrent kernel for G=%d BT=%d JU=%d wsmem=%d", G, p.BT, p.JU, (int)p.wsmem);
   return SBR_E_ARG;
 }
 
@@ -626,7 +644,7 @@ int launch_rnn_forward(sbr_model* m, const LayerDesc& L, const int32_t* len, int
     if (rc <= 0) return rc;
   }
   if (step_scan_applies(m, L.G, L.H)) return launch_rnn_forward_steps(m, L, len, B, t_max, h_last);
-  const Plan p = make_plan(m, L.G, L.H, B, false);
+  const Plan p = make_plan(m->n_sm, L.G, L.H, B, false);
   if (p.C == 0) {
     sbr_set_error(m, SBR_E_ARG, "hidden size %d is not supported by the cluster scan (max 512)", L.H);
     return SBR_E_ARG;
@@ -656,7 +674,7 @@ int launch_rnn_backward(sbr_model* m, const LayerDesc& L, const int32_t* len, in
     }
     if (step_scan_applies(m, L.G, L.H)) return launch_rnn_backward_steps(m, L, len, B, t_max, dh_last);
   }
-  const Plan p = make_plan(m, L.G, L.H, B, true);
+  const Plan p = make_plan(m->n_sm, L.G, L.H, B, true);
   if (p.C == 0) {
     sbr_set_error(m, SBR_E_ARG, "hidden size %d is not supported by the cluster scan (max 512)", L.H);
     return SBR_E_ARG;
@@ -674,4 +692,55 @@ int launch_rnn_backward(sbr_model* m, const LayerDesc& L, const int32_t* len, in
   if (L.G == 4) return dispatch<4, true>(m, p, n_tiles, a);
   if (L.G == 3) return dispatch<3, true>(m, p, n_tiles, a);
   return dispatch<1, true>(m, p, n_tiles, a);
+}
+
+// Which scan variant launch_rnn_forward / launch_rnn_backward run for one layer and batch: the same decisions in the
+// same order (tc_plan + plan_tiles, the persistent slicing, step_scan_applies, make_plan).
+extern "C" SBR_API int sbr_plan_layer_scan(const sbr_model* m, int cell, int H, int B, const int32_t* lens, int t_max,
+                                           int backward, int n_sm, const int32_t* tc_slots, int splitk_slots,
+                                           sbr_scan_plan* out) {
+  const int G = cell == SBR_CELL_LSTM ? 4 : cell == SBR_CELL_GRU ? 3 : cell == SBR_CELL_VANILLA ? 1 : 0;
+  if (!out || G == 0 || H < 1 || B < 1 || t_max < 1) return SBR_E_ARG;
+  if (!m && (n_sm < 1 || !tc_slots)) return SBR_E_ARG;
+  const ScanSwitches sw = m ? scan_switches(m) : scan_switches_from_env();
+  if (sw.multicast) return SBR_E_ARG;     // the multicast forward sizes its launches from another occupancy query
+  if (m) {
+    n_sm = m->n_sm;
+    if (cudaSetDevice(m->dev) != cudaSuccess) return SBR_E_CUDA;
+  }
+  *out = sbr_scan_plan{};
+  out->G = G;
+  const TcShape tc = tc_scan_shape(G, H);
+  if (backward ? (tc.bwd_ok && !sw.disable_tc_bwd) : tc.ok) {
+    const int slots = m ? tc_scan_slots(G, H) : tc_slots[tc.C == 8 ? 3 : tc.C == 4 ? 2 : tc.C == 2 ? 1 : 0];
+    out->family = SBR_SCAN_TC_CLUSTER;
+    out->C = tc.C; out->Hs = tc.Hs; out->MT = backward ? tc.MT : 0;
+    tc_scan_schedule(lens, B, t_max, slots, backward != 0, &out->BT, &out->launches);
+    return 0;
+  }
+  // the backward of a tcgen05-shaped layer under SBR_DISABLE_TC_BWD goes straight to the FFMA scan
+  const bool others = !backward || !tc.bwd_ok;
+  if (others && persistent_scan_applies(sw, H)) {
+    const PersistentSlicing sl = backward ? persistent_bwd_slicing(n_sm, H, B, sw.splitk,
+                                                                   sw.splitk ? (m ? persistent_splitk_slots() : splitk_slots) : 0)
+                                          : persistent_fwd_slicing(n_sm, H, B);
+    out->family = SBR_SCAN_PERSISTENT;
+    out->BT = sl.tile_rows; out->splitk = sl.splitk ? 1 : 0;
+    out->Hs = sl.owner; out->C = cdiv(H, sl.owner);
+    out->tiles_per_launch = sl.tiles_per_launch;
+    out->launches = cdiv(sl.n_tiles, sl.tiles_per_launch);
+    return 0;
+  }
+  if (others && step_scan_applies(sw, H)) {
+    out->family = SBR_SCAN_STEP;
+    out->C = 1; out->Hs = H;
+    out->launches = t_max + (backward ? 1 : 0);   // one per time step (the backward adds the initial-state step)
+    return 0;
+  }
+  const Plan p = make_plan(n_sm, G, H, B, backward != 0);
+  if (p.C == 0) return SBR_E_ARG;
+  out->family = SBR_SCAN_FFMA;
+  out->C = p.C; out->Hs = p.Hs; out->BT = p.BT; out->JU = p.JU; out->wsmem = p.wsmem ? 1 : 0;
+  out->launches = 1;
+  return 0;
 }

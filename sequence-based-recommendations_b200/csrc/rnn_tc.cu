@@ -1251,6 +1251,8 @@ TileSched plan_tiles(const int32_t* hl, int B, int t_max, int slots, float ratio
 TileSched schedule_tiles(const sbr_model* m, const TcPlan& p, int B, int t_max, float ratio8) {
   return plan_tiles(m->cur_hlen, B, t_max, resident_clusters(p), ratio8);
 }
+constexpr float TC_RATIO8_FWD = 0.71f;   // fwd: 2914 vs 4114 cycles per step (8 vs 16 rows)
+constexpr float TC_RATIO8_BWD = 0.75f;   // bwd: 4118 vs 5477 cycles per step (8 vs 16 rows)
 
 template <typename Kern>
 int launch_tc(sbr_model* m, Kern kern, const TcPlan& p, int n_tiles, const TcArgs& args, int threads, cudaStream_t stream) {
@@ -1281,6 +1283,7 @@ int launch_tc(sbr_model* m, Kern kern, const TcPlan& p, int n_tiles, const TcArg
   e = cudaLaunchKernelEx(&cfg, kern, args);
   if (e != cudaSuccess) { sbr_set_error(m, SBR_E_CUDA, "tcgen05 scan launch (C=%d) failed: %s", p.C, cudaGetErrorString(e)); return SBR_E_CUDA; }
   m->launches++;
+  m->scan_launches++;
   return 0;
 }
 
@@ -1298,7 +1301,7 @@ int launch_rnn_forward_tc(sbr_model* m, const LayerDesc& L, const int32_t* len, 
   a.len = len; a.hs = L.hs; a.cs = L.cs; a.act = L.act; a.h_last = h_last;
   a.clip = m->cfg.grad_clip; a.relu = L.relu; a.B = B; a.H = L.H; a.Hs = p.Hs; a.Kp = p.Kp; a.t_max = t_max;
   if (const char* e = getenv("SBR_TC_EXPERIMENT")) a.xflags = atoi(e);
-  const TileSched sc = schedule_tiles(m, p, B, t_max, 0.71f);   // fwd: 2914 vs 4114 cycles per step (8 vs 16 rows)
+  const TileSched sc = schedule_tiles(m, p, B, t_max, TC_RATIO8_FWD);
   const int BT = sc.BT;
   static long long* dbg = nullptr;
   if (getenv("SBR_TC_TIMELINE")) {
@@ -1357,7 +1360,7 @@ int launch_rnn_backward_tc(sbr_model* m, const LayerDesc& L, const int32_t* len,
   a.dh_last = dh_last; a.dhs = dh_last ? nullptr : L.dhs; a.dXg = L.dXg; a.dac = L.dac;
   a.g_peep = m->grads + L.peep; a.g_h_init = m->grads + L.h_init; a.g_c_init = m->grads + L.c_init;
   a.clip = m->cfg.grad_clip; a.relu = L.relu; a.B = B; a.H = L.H; a.Hs = p.Hs; a.Kp = p.Kp; a.t_max = t_max;
-  const TileSched sc = schedule_tiles(m, p, B, t_max, 0.75f);   // bwd: 4118 vs 5477 cycles per step (8 vs 16 rows)
+  const TileSched sc = schedule_tiles(m, p, B, t_max, TC_RATIO8_BWD);
   const int BT = sc.BT;
   a.g_b = m->grads + L.b;
   a.ld_p = 3;
@@ -1429,4 +1432,19 @@ extern "C" SBR_API int sbr_plan_scan_tiles(const int32_t* lens, int B, int t_max
 int tc_scan_applies(int G, int H) {
   const TcPlan p = tc_plan(G, H);
   return (p.ok && p.bwd_ok) ? 1 : 0;
+}
+
+TcShape tc_scan_shape(int G, int H) {
+  const TcPlan p = tc_plan(G, H);
+  return TcShape{p.ok, p.ok && p.bwd_ok, p.C, p.Hs, p.MT};
+}
+int tc_scan_slots(int G, int H) {
+  const TcPlan p = tc_plan(G, H);
+  return p.ok ? resident_clusters(p) : 0;
+}
+// tile height of the main launch and number of launches (the mixed tiling adds the 16-row launch on the aux stream)
+void tc_scan_schedule(const int32_t* hl, int B, int t_max, int slots, bool backward, int* tile_rows, int* n_launches) {
+  const TileSched sc = plan_tiles(hl, B, t_max, slots, backward ? TC_RATIO8_BWD : TC_RATIO8_FWD);
+  *tile_rows = sc.BT;
+  *n_launches = 1 + (sc.extra16 >= 0 ? 1 : 0);
 }

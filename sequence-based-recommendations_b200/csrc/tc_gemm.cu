@@ -809,10 +809,13 @@ int launch_gemm_tc(sbr_model* m, bool ta, bool tb, int M, int N, int K, const fl
 }
 
 // 1 when the per-step tensor-core scan handles this layer (hidden sizes beyond the cluster-resident kernels)
+int step_scan_applies(const ScanSwitches& s, int H) {
+  // H % 16: the GRU backward switches its B source (dXg | dac) at k = 2H, which must be a 32-wide chunk boundary
+  return (s.tc_gemm && s.step && H % 16 == 0 && H >= 32) ? 1 : 0;
+}
 int step_scan_applies(const sbr_model* m, int G, int H) {
   (void)G;
-  // H % 16: the GRU backward switches its B source (dXg | dac) at k = 2H, which must be a 32-wide chunk boundary
-  return (m->use_tc_gemm && m->use_step_scan && H % 16 == 0 && H >= 32) ? 1 : 0;
+  return step_scan_applies(scan_switches(m), H);
 }
 
 int launch_rnn_forward_steps(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, float* h_last) {
@@ -850,6 +853,7 @@ int launch_rnn_forward_steps(sbr_model* m, const LayerDesc& L, const int32_t* le
     else if (G == 3) rc = launch_tg<EPI_GRU_FWD>(m, a, grid);
     else rc = launch_tg<EPI_VAN_FWD>(m, a, grid);
     if (rc) return rc;
+    m->scan_launches++;
   }
   if (h_last) {
     gather_last_state_kernel<<<cdiv((int64_t)B * H, 256), 256, 0, m->stream>>>(L.hs, len, h_last, B, H, t_max);
@@ -911,6 +915,7 @@ int launch_rnn_backward_steps(sbr_model* m, const LayerDesc& L, const int32_t* l
       rc = launch_tg<EPI_INIT_GRAD>(m, a, grid);
     }
     if (rc) return rc;
+    m->scan_launches++;
   }
   return 0;
 }

@@ -1064,6 +1064,7 @@ int launch_coop(sbr_model* m, Kern kern, dim3 grid, size_t smem, const ScanArgs&
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, a);
   if (e != cudaSuccess) { sbr_set_error(m, SBR_E_CUDA, "persistent scan launch (%u x %u CTAs) failed: %s", grid.x, grid.y, cudaGetErrorString(e)); return SBR_E_CUDA; }
   m->launches++;
+  m->scan_launches++;
   return 0;
 }
 
@@ -1097,6 +1098,7 @@ int launch_cluster_coop(sbr_model* m, Kern kern, dim3 grid, dim3 cl, size_t smem
   }
   if (e != cudaSuccess) { sbr_set_error(m, SBR_E_CUDA, "split-K scan launch (%u x %u x %u CTAs) failed: %s", grid.x, grid.y, grid.z, cudaGetErrorString(e)); return SBR_E_CUDA; }
   m->launches++;
+  m->scan_launches++;
   return 0;
 }
 
@@ -1118,9 +1120,47 @@ int max_clusters(Kern kern, dim3 cl, size_t smem) {
 
 // 1 when the persistent kernels take this layer: tensor maps possible (always for arena / workspace arrays with H % 16
 // == 0), the resident forward W_hid slice fits, and the per-launch grid can be made co-resident by slicing the batch
+int persistent_scan_applies(const ScanSwitches& s, int H) {
+  return (s.tc_gemm && s.step && s.persistent && s.tma_gemm && H % 16 == 0 && H >= 32 && H <= 512) ? 1 : 0;
+}
 int persistent_scan_applies(const sbr_model* m, int G, int H) {
   (void)G;
-  return (m->use_tc_gemm && m->use_step_scan && m->use_persistent_scan && m->use_tma_gemm && H % 16 == 0 && H >= 32 && H <= 512) ? 1 : 0;
+  return persistent_scan_applies(scan_switches(m), H);
+}
+
+// shared memory of the split-K backward CTA (independent of the layer: the ring depth fills what is left)
+static size_t splitk_smem(int* look) {
+  const size_t fixed2 = (size_t)SC_ST * SC_BN * SC_KC * 8 + (size_t)SC_BN * 128 * 4 + (size_t)2 * SC_KS * SC_OWN * 128 * 4 +
+                        (size_t)2 * SC_OWN * 128 * 4 + (size_t)SC_LOOKB * SC_BN * SC_KC * 4 + 1024;
+  *look = (int)std::min<size_t>(SC_LOOK_MAX, (SC_SMEM_MAX - fixed2) / (128 * SC_KC * 4));
+  return fixed2 + (size_t)*look * 128 * SC_KC * 4;
+}
+int persistent_splitk_slots() {
+  static int slots = -1;
+  if (slots < 0) {
+    int look = 0;
+    const size_t smem2 = splitk_smem(&look);
+    slots = max_clusters(tc_scan_bwd2_kernel<4>, dim3(1, 1, SC_KS), smem2);
+  }
+  return slots;
+}
+// forward: one CTA per 8 hidden units and 128-row tile, one CTA per SM
+PersistentSlicing persistent_fwd_slicing(int n_sm, int H, int B) {
+  const int unit_ctas = cdiv(H, SC_U);
+  return PersistentSlicing{128, cdiv(B, 128), std::max(1, n_sm / unit_ctas), SC_U, false};
+}
+// backward: per 32-row tile, one 128-unit CTA (or split-K cluster of SC_KS CTAs) per 128 hidden units; split-K when at
+// least one tile's clusters are co-resident
+PersistentSlicing persistent_bwd_slicing(int n_sm, int H, int B, bool use_splitk, int splitk_slots) {
+  const int m_ctas = cdiv(H, 128);
+  PersistentSlicing s{SC_BN, cdiv(B, SC_BN), 0, 128, false};
+  if (use_splitk && splitk_slots / m_ctas >= 1) {
+    s.splitk = true;
+    s.tiles_per_launch = splitk_slots / m_ctas;
+  } else {
+    s.tiles_per_launch = std::max(1, n_sm / m_ctas);
+  }
+  return s;
 }
 
 int launch_rnn_forward_persistent(sbr_model* m, const LayerDesc& L, const int32_t* len, int B, int t_max, float* h_last) {
@@ -1153,7 +1193,7 @@ int launch_rnn_forward_persistent(sbr_model* m, const LayerDesc& L, const int32_
   const size_t smem = fixed + (size_t)a.look * 128 * SC_KC * 4;
   // batch tiles per launch: all CTAs of a launch must be co-resident (one per SM); rows are independent, so a larger
   // batch runs as several launches over slices of its tiles
-  int tiles_per_launch = std::max(1, m->n_sm / unit_ctas);
+  int tiles_per_launch = persistent_fwd_slicing(m->n_sm, H, B).tiles_per_launch;
   if (CS > 1) {
     static int slots[5] = {-1, -1, -1, -1, -1};
     if (slots[CS] < 0) slots[CS] = max_clusters(tc_scan_fwd_kernel<4>, dim3(CS, 1, 1), smem);
@@ -1198,17 +1238,14 @@ int launch_rnn_backward_persistent(sbr_model* m, const LayerDesc& L, const int32
     return 1;
   if (G == 3 && !get_tmap(&a.tmB2, L.dac, H, (uint64_t)m->T * m->B, H, SC_KC, SC_BN, true)) return 1;
   const int m_ctas0 = cdiv(H, 128), n_tiles0 = cdiv(B, SC_BN);
-  if (m->use_splitk_scan) {
+  const PersistentSlicing sl = persistent_bwd_slicing(m->n_sm, H, B, m->use_splitk_scan,
+                                                      m->use_splitk_scan ? persistent_splitk_slots() : 0);
+  if (sl.splitk) {
     // split-K clusters: KS CTAs per (hidden tile, batch tile)
-    const size_t fixed2 = (size_t)SC_ST * SC_BN * SC_KC * 8 + (size_t)SC_BN * 128 * 4 + (size_t)2 * SC_KS * SC_OWN * 128 * 4 +
-                          (size_t)2 * SC_OWN * 128 * 4 + (size_t)SC_LOOKB * SC_BN * SC_KC * 4 + 1024;
     ScanArgs v = a;
-    v.look = (int)std::min<size_t>(SC_LOOK_MAX, (SC_SMEM_MAX - fixed2) / (128 * SC_KC * 4));
-    const size_t smem2 = fixed2 + (size_t)v.look * 128 * SC_KC * 4;
-    static int slots = -1;
-    if (slots < 0) slots = max_clusters(tc_scan_bwd2_kernel<4>, dim3(1, 1, SC_KS), smem2);
-    const int tiles_per = slots / m_ctas0;      // batch tiles whose clusters are all co-resident
-    if (tiles_per >= 1) {
+    const size_t smem2 = splitk_smem(&v.look);
+    const int tiles_per = sl.tiles_per_launch;      // batch tiles whose clusters are all co-resident
+    {
       CU_TRY(m, cudaMemsetAsync(m->scan_sync, 0, (size_t)std::max(n_tiles0, cdiv(B, 128)) * sizeof(unsigned int), m->stream));
       for (int t0 = 0; t0 < n_tiles0; t0 += tiles_per) {
         const int nt = std::min(tiles_per, n_tiles0 - t0);
@@ -1228,7 +1265,7 @@ int launch_rnn_backward_persistent(sbr_model* m, const LayerDesc& L, const int32
   a.look = (int)std::min<size_t>(SC_LOOK_MAX, (SC_SMEM_MAX - fixed) / (128 * SC_KC * 4));
   const size_t smem = fixed + (size_t)a.look * 128 * SC_KC * 4;
   const int m_ctas = cdiv(H, 128), n_tiles = cdiv(B, SC_BN);
-  const int tiles_per_launch = std::max(1, m->n_sm / m_ctas);
+  const int tiles_per_launch = sl.tiles_per_launch;
   CU_TRY(m, cudaMemsetAsync(m->scan_sync, 0, (size_t)std::max(n_tiles, cdiv(B, 128)) * sizeof(unsigned int), m->stream));
   for (int t0 = 0; t0 < n_tiles; t0 += tiles_per_launch) {
     const int nt = std::min(tiles_per_launch, n_tiles - t0);
