@@ -162,6 +162,50 @@ SBR_API int sbr_scores(sbr_model* m, const int32_t* X, const float* mask, int B,
 SBR_API int sbr_topk(sbr_model* m, const int32_t* X, const float* mask, int B, const int32_t* excl_offsets,
              const int32_t* excl_ids, int k, int mode, int32_t* ids_out);
 
+/* ---- RNNCluster (neural_networks/rnn_cluster.py) ------------------------------------------ */
+/* A sampled-output RNN (BlackoutLayer, no /pop, no tanh) trained together with a soft assignment of the items to
+ * clusters: selection q = h Wc (Wc [H_last, C], no bias), P = softmax(s (q + noise)); membership rows R [N, C];
+ * cluster scores P act(s R[cells_c])^T with the same loss as the recommendation branch (rnn_cluster.py:222-251).
+ * cluster.R and cluster.W follow out.b in the parameter, gradient and optimizer arenas, so sbr_param_*, sbr_get_grad,
+ * sbr_reset_optimizer, the fused update and the one all-reduce per step cover them.  The cluster cost reaches only
+ * Wc and R, the recommendation cost only the stack and out.*: one fused update over both is exactly the reference's
+ * two updater instances (disjoint parameters, elementwise rules, equal step counters). */
+enum { SBR_CLUSTER_SOFTMAX = 0, SBR_CLUSTER_MIX = 1, SBR_CLUSTER_SIGMOID = 2 };            /* --cluster_type */
+enum { SBR_CLOSS_BLACKOUT = 0, SBR_CLOSS_CCE = 1, SBR_CLOSS_BPR = 2, SBR_CLOSS_TOP1 = 3,
+       SBR_CLOSS_BPRELU = 4, SBR_CLOSS_LIN = 5 };                                          /* --loss with --clusters */
+typedef struct sbr_cluster_config {
+  int32_t struct_size;              /* = sizeof(sbr_cluster_config), ABI guard                 */
+  int32_t n_clusters;               /* C = --clusters (>= 1)                                    */
+  int32_t cluster_type;             /* SBR_CLUSTER_*                                            */
+  int32_t loss;                     /* SBR_CLOSS_*, both branches (rnn_cluster.py:85-98)        */
+  int32_t n_cluster_samples;        /* capacity of the separate cluster samples (--c_sampling), 0 = none */
+} sbr_cluster_config;
+/* cfg->loss is ignored: the model scores its outputs linearly like the sampled models (sbr_scores / sbr_topk) */
+SBR_API int sbr_create_cluster(const sbr_config* cfg, const sbr_cluster_config* ccfg, sbr_model** out);
+/* One step of both branches.  cells = [Y_all; samples], cluster cells = [Y_all; cluster_samples] (NULL: the samples);
+ * noise [B, C] (this rank's rows) or NULL; scale = the current s.  cost and cluster_cost (may be NULL) are global means
+ * over the whole batch (the cluster cost is all-reduced with the cost). */
+SBR_API int sbr_train_step_cluster(sbr_model* m, const int32_t* X, const float* mask, const int32_t* Y_all, int n_all,
+                                   int row_offset, const int32_t* samples, int S, const int32_t* cluster_samples, int Sc,
+                                   const float* noise, float scale, int B, float* cost, float* cluster_cost);
+/* Validation test function (rnn_cluster.py:327-355): score1 = softmax(h W + b) with the excluded ids multiplied by 0,
+ * c = argmax(h Wc), score2 = score1 * hard[:, c] (hard = softmax / clip(softmax + sigmoid) / sigmoid of 100 R);
+ * per row the top-k of both scores, c, and n_used = sum_n hard[n, c].  k <= 64. */
+SBR_API int sbr_cluster_test_topk(sbr_model* m, const int32_t* X, const float* mask, int B, const int32_t* excl_offsets,
+                                  const int32_t* excl_ids, int k, int32_t* ids_full, int32_t* ids_cluster,
+                                  int32_t* selected, float* n_used);
+/* prepare_tests (rnn_cluster.py:461-487): item n belongs to every cluster j with R[n, j] > 0, an item without a
+ * positive entry to the first arg-max of its row; clusters list their items in ascending id.  Built on the device and
+ * kept there; sizes [C] (may be NULL) receives the cluster sizes. */
+SBR_API int sbr_cluster_build(sbr_model* m, int32_t* sizes);
+/* top_k_recommendations (rnn_cluster.py:293-322).  use_clusters: c = argmax(h Wc), only the items of cluster c are
+ * scored (h W[:, items] + b[items]), excluded ids are -inf, ids_out[b, :min(k, |c|)] best first (-1 beyond),
+ * n_out[b] = |c|, selected_out[b] = c (may be NULL).  use_clusters = 0: the whole catalog, n_out[b] = n_items.  The
+ * work scales with sum_b |cluster(b)| * H_last.  Needs sbr_cluster_build after the last parameter change. */
+SBR_API int sbr_cluster_topk(sbr_model* m, const int32_t* X, const float* mask, int B, const int32_t* excl_offsets,
+                             const int32_t* excl_ids, int k, int32_t* ids_out, int32_t* n_out, int32_t* selected_out,
+                             int use_clusters);
+
 /* ---- measurement ------------------------------------------------------------------------ */
 #define SBR_N_STAGES 9
 SBR_API const char* sbr_stage_name(int i);            /* "h2d","gather","rnn_fwd","output","rnn_bwd","wgrad","scatter","allreduce","optimizer" */

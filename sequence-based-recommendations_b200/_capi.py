@@ -22,6 +22,8 @@ SBR_N_STAGES = 9
 CELLS = {"LSTM": 0, "GRU": 1, "Vanilla": 2}
 LOSSES = {"CCE": 0, "BPR": 1, "BPRI": 2, "TOP1": 3, "Blackout": 4, "hinge": 5, "logit": 6, "logsig": 7}
 UPDATERS = {"adam": 0, "adagrad": 1, "adadelta": 2, "rmsprop": 3, "nesterov": 4}
+CLUSTER_TYPES = {"softmax": 0, "mix": 1, "sigmoid": 2}
+CLUSTER_LOSSES = {"Blackout": 0, "CCE": 1, "BPR": 2, "TOP1": 3, "BPRelu": 4, "lin": 5}
 STATUS = {0: "SBR_OK", -1: "SBR_E_ARG", -2: "SBR_E_CUDA", -3: "SBR_E_NCCL", -4: "SBR_E_MASK",
           -5: "SBR_E_RANGE", -6: "SBR_E_NOGPU"}
 
@@ -45,6 +47,11 @@ class SbrConfig(C.Structure):
         ("global_batch", C.c_int32), ("n_slots", C.c_int32), ("bidirectional", C.c_int32),
         ("nccl_id", C.c_uint8 * SBR_NCCL_ID_BYTES),
     ]
+
+
+class SbrClusterConfig(C.Structure):
+    _fields_ = [("struct_size", C.c_int32), ("n_clusters", C.c_int32), ("cluster_type", C.c_int32), ("loss", C.c_int32),
+                ("n_cluster_samples", C.c_int32)]
 
 
 class SbrScanPlan(C.Structure):
@@ -86,6 +93,12 @@ SIGNATURES = {
     "sbr_synchronize": (C.c_int, [_P, _f32p]),
     "sbr_scores": (C.c_int, [_P, _i32p, _f32p, C.c_int, C.c_int, _f32p]),
     "sbr_topk": (C.c_int, [_P, _i32p, _f32p, C.c_int, _i32p, _i32p, C.c_int, C.c_int, _i32p]),
+    "sbr_create_cluster": (C.c_int, [C.POINTER(SbrConfig), C.POINTER(SbrClusterConfig), C.POINTER(_P)]),
+    "sbr_train_step_cluster": (C.c_int, [_P, _i32p, _f32p, _i32p, C.c_int, C.c_int, _i32p, C.c_int, _i32p, C.c_int, _f32p,
+                                         C.c_float, C.c_int, _f32p, _f32p]),
+    "sbr_cluster_test_topk": (C.c_int, [_P, _i32p, _f32p, C.c_int, _i32p, _i32p, C.c_int, _i32p, _i32p, _i32p, _f32p]),
+    "sbr_cluster_build": (C.c_int, [_P, _i32p]),
+    "sbr_cluster_topk": (C.c_int, [_P, _i32p, _f32p, C.c_int, _i32p, _i32p, C.c_int, _i32p, _i32p, _i32p, C.c_int]),
     "sbr_stage_name": (C.c_char_p, [C.c_int]),
     "sbr_set_profiling": (C.c_int, [_P, C.c_int]),
     "sbr_stage_times": (C.c_int, [_P, _f32p]),
@@ -181,7 +194,9 @@ class Engine(object):
                  embedding=0, n_extra_ids=0, ids_per_step=1, n_samples=32, last_layer_tanh=False,
                  updater="adam", lr=1e-3, rho=0.9, beta1=0.9, beta2=0.999, grad_clip=100.0,
                  regularization=0.0, device=0, n_ranks=1, rank=0, nccl_id=None, global_batch=0,
-                 n_slots=1, math_mode=0, bidirectional=False):
+                 n_slots=1, math_mode=0, bidirectional=False, clusters=None):
+        """clusters: None, or dict(n_clusters, cluster_type, loss, n_cluster_samples) for an RNNCluster handle
+        (sbr_create_cluster); `loss` is then ignored."""
         self.lib = load_library()
         cfg = SbrConfig()
         cfg.struct_size = C.sizeof(SbrConfig)
@@ -194,7 +209,8 @@ class Engine(object):
             cfg.layers[i] = int(h)
         cfg.n_items, cfg.n_extra_ids, cfg.ids_per_step = int(n_items), int(n_extra_ids), int(ids_per_step)
         cfg.embedding, cfg.max_length, cfg.batch_size = int(embedding), int(max_length), int(batch_size)
-        cfg.loss, cfg.n_samples, cfg.last_layer_tanh = LOSSES[loss], int(n_samples), int(bool(last_layer_tanh))
+        cfg.loss = LOSSES["Blackout"] if clusters else LOSSES[loss]
+        cfg.n_samples, cfg.last_layer_tanh = int(n_samples), int(bool(last_layer_tanh))
         cfg.updater = UPDATERS[updater]
         cfg.lr, cfg.rho, cfg.beta1, cfg.beta2 = lr, rho, beta1, beta2
         cfg.grad_clip, cfg.regularization = grad_clip, regularization
@@ -212,7 +228,19 @@ class Engine(object):
         self.ids_per_step = int(ids_per_step)
         self.n_samples = int(n_samples)
         self._h = _P()
-        rc = self.lib.sbr_create(C.byref(cfg), C.byref(self._h))
+        self.n_clusters = 0
+        if clusters:
+            cc = SbrClusterConfig()
+            cc.struct_size = C.sizeof(SbrClusterConfig)
+            cc.n_clusters = int(clusters["n_clusters"])
+            cc.cluster_type = CLUSTER_TYPES[clusters.get("cluster_type", "mix")]
+            cc.loss = CLUSTER_LOSSES[clusters.get("loss", "Blackout")]
+            cc.n_cluster_samples = max(0, int(clusters.get("n_cluster_samples", 0)))
+            self.n_clusters = int(cc.n_clusters)
+            self.ccfg = cc
+            rc = self.lib.sbr_create_cluster(C.byref(cfg), C.byref(cc), C.byref(self._h))
+        else:
+            rc = self.lib.sbr_create(C.byref(cfg), C.byref(self._h))
         if rc != 0:
             self._h = None
             raise SbrError(rc, self.lib.sbr_last_error(None).decode())
@@ -314,6 +342,23 @@ class Engine(object):
                                                     _ptr(pop, _f32p), B, C.byref(cost)))
         return np.float32(cost.value)
 
+    def train_step_cluster(self, X, mask, Y, samples, cluster_samples=None, noise=None, scale=1.0, Y_all=None,
+                           row_offset=0):
+        """RNNCluster step; returns (cost, cluster_cost).  noise: [B, n_clusters] of this rank's rows, or None."""
+        X, mask, B = self._xm(X, mask)
+        Y_all = _i32(Y if Y_all is None else Y_all)
+        samples = _i32(samples)
+        cs = None if cluster_samples is None else _i32(cluster_samples)
+        nz = None if noise is None else _f32(noise)
+        if nz is not None and nz.shape != (B, self.n_clusters):
+            raise ValueError("noise must be [B, %d]" % self.n_clusters)
+        cost, ccost = C.c_float(0), C.c_float(0)
+        self._check(self.lib.sbr_train_step_cluster(
+            self._h, _ptr(X, _i32p), _ptr(mask, _f32p), _ptr(Y_all, _i32p), len(Y_all), int(row_offset),
+            _ptr(samples, _i32p), len(samples), None if cs is None else _ptr(cs, _i32p), 0 if cs is None else len(cs),
+            None if nz is None else _ptr(nz, _f32p), float(scale), B, C.byref(cost), C.byref(ccost)))
+        return np.float32(cost.value), np.float32(ccost.value)
+
     def train_step_margin_dense(self, X, mask, Ymat, weight):
         X, mask, B = self._xm(X, mask)
         Ymat, weight = _f32(Ymat), _f32(weight)
@@ -397,6 +442,46 @@ class Engine(object):
         self._check(self.lib.sbr_topk(self._h, _ptr(X, _i32p), _ptr(mask, _f32p), B, off_p, ids_p, int(k), mode,
                                       _ptr(out, _i32p)))
         return out
+
+    @staticmethod
+    def _ragged(exclude, B):
+        if exclude is None:
+            return None, None, None
+        off = np.zeros(B + 1, dtype=np.int32)
+        off[1:] = np.cumsum([len(e) for e in exclude])
+        flat = [i for e in exclude for i in e]
+        ids = _i32(flat if flat else [0])
+        return (off, ids), _ptr(off, _i32p), _ptr(ids, _i32p)
+
+    def cluster_test_topk(self, X, mask, k=10, exclude=None):
+        """Validation test function of RNNCluster: (ids_full [B,k], ids_cluster [B,k], selected [B], n_used [B])."""
+        X, mask, B = self._xm(X, mask)
+        keep, off_p, ids_p = self._ragged(exclude, B)
+        full = np.empty((B, k), dtype=np.int32)
+        clus = np.empty((B, k), dtype=np.int32)
+        sel = np.empty(B, dtype=np.int32)
+        used = np.empty(B, dtype=np.float32)
+        self._check(self.lib.sbr_cluster_test_topk(self._h, _ptr(X, _i32p), _ptr(mask, _f32p), B, off_p, ids_p, int(k),
+                                                   _ptr(full, _i32p), _ptr(clus, _i32p), _ptr(sel, _i32p),
+                                                   _ptr(used, _f32p)))
+        return full, clus, sel, used
+
+    def cluster_build(self):
+        """Hard clusters from cluster.R on the device; returns the cluster sizes."""
+        sizes = np.empty(self.n_clusters, dtype=np.int32)
+        self._check(self.lib.sbr_cluster_build(self._h, _ptr(sizes, _i32p)))
+        return sizes
+
+    def cluster_topk(self, X, mask, k=10, exclude=None, use_clusters=True):
+        """(ids [B,k] with -1 past min(k, |cluster|), n [B], selected [B])."""
+        X, mask, B = self._xm(X, mask)
+        keep, off_p, ids_p = self._ragged(exclude, B)
+        ids = np.empty((B, k), dtype=np.int32)
+        n = np.empty(B, dtype=np.int32)
+        sel = np.empty(B, dtype=np.int32)
+        self._check(self.lib.sbr_cluster_topk(self._h, _ptr(X, _i32p), _ptr(mask, _f32p), B, off_p, ids_p, int(k),
+                                              _ptr(ids, _i32p), _ptr(n, _i32p), _ptr(sel, _i32p), int(bool(use_clusters))))
+        return ids, n, sel
 
     # -- measurement ----------------------------------------------------------------------------
     def set_profiling(self, on):

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsbr_b200.so")
-SOURCES = ["model.cu", "gather_scatter.cu", "rnn_cluster.cu", "rnn_tc.cu", "wgrad_tc.cu", "tc_gemm.cu", "tc_scan.cu", "gemm.cu", "loss.cu", "optim.cu"]
+SOURCES = ["model.cu", "gather_scatter.cu", "rnn_cluster.cu", "rnn_tc.cu", "wgrad_tc.cu", "tc_gemm.cu", "tc_scan.cu", "gemm.cu", "loss.cu", "optim.cu", "cluster.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--use_fast_math=false",

@@ -158,6 +158,37 @@ struct sbr_model {
   float* w_neg = nullptr;
   float* def_tgt = nullptr;
   int tgt_cap = 0;
+  // RNNCluster (sbr_create_cluster): cluster.R [N, C] and cluster.W [H_last, C] follow out.b in the arenas
+  int n_clusters = 0;         // 0: not a cluster model
+  int cluster_type = 0;       // SBR_CLUSTER_*
+  int cluster_loss = 0;       // sampling_loss_kernel code of the SBR_CLOSS_* of both branches
+  int n_csamples = 0;         // capacity of the cluster-sample vector
+  int64_t cl_R = 0, cl_W = 0; // arena offsets
+  int32_t* ccells = nullptr;  // [n_all + Sc] cluster cells = [Y_all; cluster samples]
+  float* cq = nullptr;        // [B, C] h Wc
+  float* cnoise = nullptr;    // [B, C] selection noise of this rank's rows
+  float* cP = nullptr;        // [B, C] scaled selection softmax
+  float* cdP = nullptr;       // [B, C]
+  float* cdq = nullptr;       // [B, C]
+  float* cM = nullptr;        // [n_all + Sc, C] membership rows
+  float* cdM = nullptr;
+  float* cS = nullptr;        // [B, n_all + Sc] cluster scores, then their gradient
+  float* crow_loss = nullptr; // [B]
+  int32_t* csel = nullptr;    // [B] selected cluster per row
+  float* cnused = nullptr;    // [B] items of the hard column per row
+  int32_t* cperm = nullptr;   // [B] rows grouped by selected cluster
+  float* ch_sorted = nullptr; // [B, H_last] final states in that order
+  float* clse = nullptr;      // [N] logsumexp of 100 R per item
+  float* logits2 = nullptr;   // [B, N] cluster-weighted test scores (allocated on first use)
+  // item CSR of the hard clusters (sbr_cluster_build), device resident
+  int32_t* cl_off = nullptr;  // [C + 1]
+  int32_t* cl_items = nullptr;
+  int32_t* cl_fb = nullptr;   // [N] fallback cluster of an item without a positive entry (-1: has one)
+  int32_t* cl_cnt = nullptr;  // [chunks, C] counts, then offsets inside the cluster
+  float* cl_Wg = nullptr;     // [max cluster size, H_last] gathered output rows of one cluster
+  std::vector<int32_t> cl_hoff;   // host copy of cl_off (empty: not built)
+  int64_t cl_cap_items = 0;   // allocated lengths of cl_items / rows of cl_Wg
+  int cl_cap_rows = 0;
   // top-k
   int32_t* excl_off = nullptr;
   int32_t* excl_ids = nullptr;
@@ -311,3 +342,21 @@ int launch_topk(sbr_model* m, float* scores, int ld, int B, int N, const int32_t
 
 // optim.cu
 int launch_optimizer(sbr_model* m);
+
+// sampling_loss_kernel codes used only by the cluster model (never accepted by sbr_create): the sampled softmax
+// cross-entropy, the leaky-rectified BPR and the linear loss of rnn_cluster.py:158-175
+enum { SBR_LK_SCCE = 100, SBR_LK_BPRELU = 101, SBR_LK_LIN = 102 };
+
+// cluster.cu : the cluster branch of RNNCluster (rnn_cluster.py:232-251) and its test paths
+int launch_cluster_select(sbr_model* m, const float* q, const float* noise, int B, int C, float scale, float* P);
+int launch_cluster_members(sbr_model* m, const float* R, const int32_t* cells, int n, int C, int type, float scale, float* M);
+int launch_cluster_dq(sbr_model* m, const float* P, const float* dP, int B, int C, float scale, float* dq);
+int launch_cluster_dR(sbr_model* m, const float* R, const int32_t* cells, int n, int C, int type, float scale,
+                      const float* dM, float* gR);
+int launch_cluster_hard(sbr_model* m, const float* scores, int ld, const float* q, const float* R, int B, int N, int C,
+                        int type, float* scores2, int32_t* sel, float* n_used);
+int launch_cluster_argmax(sbr_model* m, const float* q, int B, int C, int32_t* sel);
+int launch_cluster_csr(sbr_model* m, const float* R, int N, int C);    // fallback, counts, m->cl_off
+int launch_cluster_fill(sbr_model* m, const float* R, int N, int C);   // m->cl_items (sized from m->cl_off[C])
+int launch_cluster_row_topk(sbr_model* m, float* scores, int ld, int B, const int32_t* perm, const int32_t* sel,
+                            const float* bias, const int32_t* excl_off, const int32_t* excl_ids, int k, int32_t* ids_out);

@@ -109,7 +109,10 @@ __global__ void add_bias_rows_kernel(float* __restrict__ logits, int ld, const f
 }
 
 // Sampling losses.  Columns [0, n_all) are the targets of the whole global batch, [n_all, n_all+S)
-// the shared negative samples; the positive of local row b is column row_offset + b.
+// the shared negative samples; the positive of local row b is column row_offset + b.  The cluster model
+// (rnn_cluster.py:151-180) passes pop = NULL (unit weights), bias_cells = NULL for its cluster scores, and three more
+// codes: SBR_LK_SCCE (-log softmax over the B+S columns, no negative term), SBR_LK_BPRELU (leaky_rectify(d + 0.5),
+// leakiness 0.01, Theano slope 0.505 at 0) and SBR_LK_LIN (sum of the negatives minus the positive, not a mean).
 __global__ void __launch_bounds__(LT) sampling_loss_kernel(int loss, int tanh_out, float* __restrict__ A, int ld,
                                                             const float* __restrict__ bias_cells,
                                                             const float* __restrict__ pop, int n_all, int row_offset,
@@ -119,11 +122,12 @@ __global__ void __launch_bounds__(LT) sampling_loss_kernel(int loss, int tanh_ou
   const int Ccols = n_all + S;
   float* row = A + (int64_t)b * ld;
   const int pc = row_offset + b;
-  const float scale = inv_gb / pop[b];
-  if (loss == SBR_LOSS_BLACKOUT) {
+  const float scale = pop ? inv_gb / pop[b] : inv_gb;
+  if (loss == SBR_LOSS_BLACKOUT || loss == SBR_LK_SCCE) {
+    const bool negs = loss == SBR_LOSS_BLACKOUT;
     float mx = -CUDART_INF_F;
     for (int n = threadIdx.x; n < Ccols; n += LT) {
-      const float z = row[n] + bias_cells[n];
+      const float z = row[n] + (bias_cells ? bias_cells[n] : 0.f);
       row[n] = z;
       mx = fmaxf(mx, z);
     }
@@ -137,7 +141,7 @@ __global__ void __launch_bounds__(LT) sampling_loss_kernel(int loss, int tanh_ou
     for (int n = threadIdx.x; n < Ccols; n += LT) {
       const float p = expf(row[n] - mx) * inv;
       if (n == pc) { lpart += -logf(p); gp += -1.f; }           // g * p = -1
-      if (n >= n_all) { lpart += -logf(1.f - p); gp += p / (1.f - p); }
+      if (negs && n >= n_all) { lpart += -logf(1.f - p); gp += p / (1.f - p); }
     }
     const float l = block_sum(lpart, sh);
     const float gdot = block_sum(gp, sh);
@@ -147,13 +151,13 @@ __global__ void __launch_bounds__(LT) sampling_loss_kernel(int loss, int tanh_ou
       const float p = expf(row[n] - mx) * inv;
       float g = 0.f;
       if (n == pc) g += -1.f / p;
-      if (n >= n_all) g += 1.f / (1.f - p);
+      if (negs && n >= n_all) g += 1.f / (1.f - p);
       row[n] = p * (g - gdot) * scale;
     }
     return;
   }
-  // BPR / BPRI / TOP1
-  float posv = row[pc] + bias_cells[pc];
+  // BPR / BPRI / TOP1 (and the cluster model's BPRelu / lin)
+  float posv = row[pc] + (bias_cells ? bias_cells[pc] : 0.f);
   if (tanh_out) posv = tanhf(posv);
   __syncthreads();
   float lpart = 0.f, gsum = 0.f;
@@ -161,13 +165,19 @@ __global__ void __launch_bounds__(LT) sampling_loss_kernel(int loss, int tanh_ou
   for (int n = threadIdx.x; n < Ccols; n += LT) {
     float out = 0.f;
     if (n >= n_all) {
-      float v = row[n] + bias_cells[n];
+      float v = row[n] + (bias_cells ? bias_cells[n] : 0.f);
       if (tanh_out) v = tanhf(v);
       const float d = v - posv;
       const float sd = sigm(d);
       float gd, gn = 0.f;
       if (loss == SBR_LOSS_BPR) { lpart += softplus(d) * invS; gd = sd * invS; }
       else if (loss == SBR_LOSS_BPRI) { lpart += (fminf(d, 0.f) - log1pf(expf(-fabsf(d)))) * invS; gd = (1.f - sd) * invS; }
+      else if (loss == SBR_LK_BPRELU) {
+        // Theano relu(x, a) = 0.5 (1 + a) x + 0.5 (1 - a) |x|: slope 1 / 0.505 / 0.01 for x > 0 / = 0 / < 0
+        const float x = d + 0.5f;
+        lpart += (x > 0.f ? x : 0.01f * x) * invS;
+        gd = (x > 0.f ? 1.f : (x == 0.f ? 0.505f : 0.01f)) * invS;
+      } else if (loss == SBR_LK_LIN) { lpart += v; gd = 0.f; gn = 1.f; }   // the positive is handled below
       else {
         const float sn = sigm(v * v);
         lpart += (sd + sn) * invS;
@@ -183,8 +193,8 @@ __global__ void __launch_bounds__(LT) sampling_loss_kernel(int loss, int tanh_ou
   const float l = block_sum(lpart, sh);
   const float gs = block_sum(gsum, sh);
   if (threadIdx.x == 0) {
-    row_loss[b] = l * scale;
-    float dp = -gs * scale;
+    row_loss[b] = (loss == SBR_LK_LIN ? l - posv : l) * scale;
+    float dp = (loss == SBR_LK_LIN ? -1.f : -gs) * scale;
     if (tanh_out) dp *= (1.f - posv * posv);
     row[pc] = dp;
   }

@@ -247,6 +247,14 @@ static int build_layout(sbr_model* m) {
   m->P += (int64_t)m->N * m->H_last + m->N;
   add_view(m, "out.W", 2, m->H_last, m->N, m->out_WT, m->H_last, m->N, m->H_last, /*transposed=*/true);
   add_view(m, "out.b", 1, m->N, 1, m->out_b, 1, m->N, m->N);
+  if (m->n_clusters > 0) {   // RNNCluster: membership rows, then the selection layer (rnn_cluster.py:235,241)
+    const int C = m->n_clusters;
+    m->cl_R = take(off, (int64_t)m->N * C);
+    m->cl_W = take(off, (int64_t)m->H_last * C);
+    m->P += (int64_t)m->N * C + (int64_t)m->H_last * C;
+    add_view(m, "cluster.R", 2, m->N, C, m->cl_R, m->N, C, C);
+    add_view(m, "cluster.W", 2, m->H_last, C, m->cl_W, m->H_last, C, C);
+  }
   m->P_pad = round_up(off, 4);
   m->cost_slot = m->P_pad;   // just past the optimised range, still inside the all-reduced range
   return 0;
@@ -265,6 +273,9 @@ extern "C" void sbr_destroy(sbr_model* m) {
   for (BatchSlot& s : m->slots) { F(s.X); F(s.len); F(s.Y); F(s.pop); }
   F(m->emb_out); F(m->demb); F(m->h_last); F(m->dh_last); F(m->logits); F(m->row_loss); F(m->WhidT); F(m->step_carry); F(m->step_dcs); F(m->step_dpe); F(m->scan_sync); F(m->ds_off); F(m->ds_ids); F(m->ds_rows); F(m->wg_list); F(m->X_rev); F(m->emb_out_rv); F(m->demb_rv); F(m->cat_al); F(m->cat_rv); F(m->dcat_al); F(m->dcat_rv); F(m->h_last_dir); F(m->dh_last_dir);
   F(m->mY); F(m->mW); F(m->cells); F(m->Wc); F(m->dWc); F(m->bc);
+  F(m->ccells); F(m->cq); F(m->cnoise); F(m->cP); F(m->cdP); F(m->cdq); F(m->cM); F(m->cdM); F(m->cS); F(m->crow_loss);
+  F(m->csel); F(m->cnused); F(m->cperm); F(m->ch_sorted); F(m->clse); F(m->logits2);
+  F(m->cl_off); F(m->cl_items); F(m->cl_fb); F(m->cl_cnt); F(m->cl_Wg);
   F(m->tgt_off); F(m->tgt_ids); F(m->w_neg); F(m->def_tgt); F(m->excl_off); F(m->excl_ids); F(m->topk_ids);
   if (m->h_len) cudaFreeHost(m->h_len);
   if (m->h_cost) cudaFreeHost(m->h_cost);
@@ -420,7 +431,7 @@ static int create_impl(sbr_model* m) {
       if ((rc = dev_alloc(m, &m->demb_rv, TB * m->K * m->E))) return rc;
     }
   }
-  const bool sampled = c.loss >= SBR_LOSS_BPR && c.loss <= SBR_LOSS_BLACKOUT;
+  const bool sampled = (c.loss >= SBR_LOSS_BPR && c.loss <= SBR_LOSS_BLACKOUT) || m->n_clusters > 0;
   const bool margin = c.loss >= SBR_LOSS_HINGE;
   const size_t n_cells = (size_t)m->global_batch + std::max(1, c.n_samples);
   // rows padded to a multiple of 4 floats: 16-byte row pitch, so the score matrix can be a TMA operand of the gradient GEMMs
@@ -431,6 +442,27 @@ static int create_impl(sbr_model* m) {
     if ((rc = dev_alloc(m, &m->Wc, n_cells * m->H_last))) return rc;
     if ((rc = dev_alloc(m, &m->dWc, n_cells * m->H_last))) return rc;
     if ((rc = dev_alloc(m, &m->bc, 2 * n_cells))) return rc;
+  }
+  if (m->n_clusters > 0) {
+    const size_t C = m->n_clusters, ncc = (size_t)m->global_batch + m->n_csamples, H = m->H_last;
+    if ((rc = dev_alloc(m, &m->ccells, ncc))) return rc;
+    if ((rc = dev_alloc(m, &m->cq, B * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cnoise, B * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cP, B * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cdP, B * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cdq, B * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cM, ncc * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cdM, ncc * C))) return rc;
+    if ((rc = dev_alloc(m, &m->cS, B * (size_t)round_up(ncc, 4)))) return rc;
+    if ((rc = dev_alloc(m, &m->crow_loss, B))) return rc;
+    if ((rc = dev_alloc(m, &m->csel, B))) return rc;
+    if ((rc = dev_alloc(m, &m->cnused, B))) return rc;
+    if ((rc = dev_alloc(m, &m->cperm, B))) return rc;
+    if ((rc = dev_alloc(m, &m->ch_sorted, B * H))) return rc;
+    if ((rc = dev_alloc(m, &m->clse, m->N))) return rc;
+    if ((rc = dev_alloc(m, &m->cl_off, C + 1))) return rc;
+    if ((rc = dev_alloc(m, &m->cl_fb, m->N))) return rc;
+    if ((rc = dev_alloc(m, &m->cl_cnt, (size_t)cdiv(m->N, 256) * C))) return rc;
   }
   if (margin) {
     // the dense [B, n_items] target / weight matrices of the reference exist only for callers of the dense entry point
@@ -481,7 +513,30 @@ static int create_impl(sbr_model* m) {
   return 0;
 }
 
-extern "C" int sbr_create(const sbr_config* cfg, sbr_model** out) {
+static int create_model(const sbr_config* cfg, const sbr_cluster_config* ccfg, sbr_model** out);
+
+extern "C" int sbr_create(const sbr_config* cfg, sbr_model** out) { return create_model(cfg, nullptr, out); }
+
+extern "C" int sbr_create_cluster(const sbr_config* cfg, const sbr_cluster_config* ccfg, sbr_model** out) {
+  if (!cfg || !ccfg || !out) { sbr_set_error(nullptr, SBR_E_ARG, "null argument"); return SBR_E_ARG; }
+  *out = nullptr;
+  if (ccfg->struct_size != (int32_t)sizeof(sbr_cluster_config)) {
+    sbr_set_error(nullptr, SBR_E_ARG, "sbr_cluster_config.struct_size %d != %zu (ABI mismatch)", ccfg->struct_size, sizeof(sbr_cluster_config));
+    return SBR_E_ARG;
+  }
+  auto bad = [&](const char* what) { sbr_set_error(nullptr, SBR_E_ARG, "unsupported cluster configuration: %s", what); return SBR_E_ARG; };
+  if (ccfg->n_clusters < 1) return bad("n_clusters must be >= 1");
+  if (ccfg->cluster_type < SBR_CLUSTER_SOFTMAX || ccfg->cluster_type > SBR_CLUSTER_SIGMOID) return bad("cluster_type");
+  if (ccfg->loss < SBR_CLOSS_BLACKOUT || ccfg->loss > SBR_CLOSS_LIN) return bad("loss");
+  if (ccfg->n_cluster_samples < 0) return bad("n_cluster_samples");
+  if (cfg->n_samples < 1) return bad("n_samples must be >= 1");
+  sbr_config c = *cfg;
+  c.loss = SBR_LOSS_BLACKOUT;   // linear outputs, sampled-column buffers; the cluster loss is kept apart
+  c.last_layer_tanh = 0;
+  return create_model(&c, ccfg, out);
+}
+
+static int create_model(const sbr_config* cfg, const sbr_cluster_config* ccfg, sbr_model** out) {
   if (!cfg || !out) { sbr_set_error(nullptr, SBR_E_ARG, "null argument"); return SBR_E_ARG; }
   *out = nullptr;
   if (cfg->struct_size != (int32_t)sizeof(sbr_config)) {
@@ -513,6 +568,13 @@ extern "C" int sbr_create(const sbr_config* cfg, sbr_model** out) {
   m->n_in = cfg->n_items + cfg->n_extra_ids; m->E = cfg->embedding; m->L = cfg->n_layers;
   m->nd = cfg->bidirectional ? 2 : 1;
   m->global_batch = cfg->global_batch > 0 ? cfg->global_batch : cfg->batch_size * cfg->n_ranks;
+  if (ccfg) {
+    static const int kcode[] = {SBR_LOSS_BLACKOUT, SBR_LK_SCCE, SBR_LOSS_BPR, SBR_LOSS_TOP1, SBR_LK_BPRELU, SBR_LK_LIN};
+    m->n_clusters = ccfg->n_clusters;
+    m->cluster_type = ccfg->cluster_type;
+    m->cluster_loss = kcode[ccfg->loss];
+    m->n_csamples = ccfg->n_cluster_samples > 0 ? ccfg->n_cluster_samples : cfg->n_samples;
+  }
   const int rc = create_impl(m);
   if (rc != 0) {
     g_create_error = m->err;
@@ -983,7 +1045,8 @@ static int finish_step(sbr_model* m, float* cost) {
   }
   stage_mark(m, 7);
   if (m->nccl_comm) {
-    ncclResult_t r = g_nccl.AllReduce(m->grads, m->grads, (size_t)m->P_pad + 1, ncclFloat, ncclSum,
+    // the cost slot rides along (the cluster model's second cost in the slot after it)
+    ncclResult_t r = g_nccl.AllReduce(m->grads, m->grads, (size_t)m->P_pad + (m->n_clusters > 0 ? 2 : 1), ncclFloat, ncclSum,
                                       (ncclComm_t)m->nccl_comm, m->stream);
     if (r != ncclSuccess) {
       sbr_set_error(m, SBR_E_NCCL, "ncclAllReduce: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?");
@@ -992,7 +1055,7 @@ static int finish_step(sbr_model* m, float* cost) {
   }
   stage_mark(m, 8);
   if (cost && !m->cost_early)
-    CU_TRY(m, cudaMemcpyAsync(m->h_cost, m->grads + m->cost_slot, sizeof(float), cudaMemcpyDeviceToHost, m->stream));
+    CU_TRY(m, cudaMemcpyAsync(m->h_cost, m->grads + m->cost_slot, (m->n_clusters > 0 ? 2 : 1) * sizeof(float), cudaMemcpyDeviceToHost, m->stream));
   if (!m->skip_update)
     if ((rc = launch_optimizer(m))) return rc;
   stage_mark(m, 9);
@@ -1073,12 +1136,15 @@ extern "C" int sbr_synchronize(sbr_model* m, float* last_cost) {
   return 0;
 }
 
+static int sampled_output(sbr_model* m, int loss, bool tanh_out, const float* pop, int B, int n_all, int row_offset, int S,
+                          float inv_gb);
+
 extern "C" int sbr_train_step_sampled(sbr_model* m, const int32_t* X, const float* mask, const int32_t* Y_all,
                                       int n_all, int row_offset, const int32_t* samples, int S, const float* pop,
                                       int B, float* cost) {
   CHECK_STICKY(m);
   const int loss = m->cfg.loss;
-  if (loss < SBR_LOSS_BPR || loss > SBR_LOSS_BLACKOUT) { sbr_set_error(m, SBR_E_ARG, "model was not created with a sampling loss"); return SBR_E_ARG; }
+  if (loss < SBR_LOSS_BPR || loss > SBR_LOSS_BLACKOUT || m->n_clusters > 0) { sbr_set_error(m, SBR_E_ARG, "model was not created with a sampling loss"); return SBR_E_ARG; }
   if (!Y_all || !samples || !pop || S < 1 || S > std::max(1, m->cfg.n_samples) || n_all < B || n_all > m->global_batch ||
       row_offset < 0 || row_offset + B > n_all) {
     sbr_set_error(m, SBR_E_ARG, "bad sampled-step arguments (S=%d n_all=%d row_offset=%d B=%d)", S, n_all, row_offset, B);
@@ -1100,22 +1166,31 @@ extern "C" int sbr_train_step_sampled(sbr_model* m, const int32_t* X, const floa
   CU_TRY(m, cudaStreamSynchronize(m->stream));
   const float inv_gb = 1.f / (float)(m->cfg.global_batch > 0 ? m->cfg.global_batch : s.B * m->cfg.n_ranks);
   if ((rc = forward_stack(m, s))) return rc;
+  if ((rc = sampled_output(m, loss, m->cfg.last_layer_tanh != 0, s.pop, B, n_all, row_offset, S, inv_gb))) return rc;
+  stage_mark(m, 4);
+  if ((rc = backward_stack(m, s))) return rc;
+  return finish_step(m, cost);
+}
+
+// BlackoutLayer of the sampled models on the gathered columns m->cells = [Y_all; samples]: scores, loss (into the
+// cost slot), the gradients of the gathered output rows / bias and m->dh_last
+static int sampled_output(sbr_model* m, int loss, bool tanh_out, const float* pop, int B, int n_all, int row_offset, int S,
+                          float inv_gb) {
+  int rc;
+  const int nc = n_all + S;
   const int H = m->H_last;
   const int ldc = (int)round_up(nc, 4);      // padded row pitch of the [B, n_all + S] score matrix
   float* bcg = m->bc + nc;   // gradient of the gathered bias entries
   // BlackoutLayer: scores of the gathered columns only (sparse_lstm.py:41-54)
   if ((rc = launch_gather_table_rows(m, m->params + m->out_WT, m->params + m->out_b, m->cells, nc, H, m->Wc, m->bc))) return rc;
   if ((rc = launch_gemm(m, false, true, B, nc, H, m->h_last, H, m->Wc, H, m->logits, ldc, 1.f, 0.f))) return rc;
-  if ((rc = launch_sampling_loss(m, loss, m->cfg.last_layer_tanh != 0, m->logits, ldc, m->bc, s.pop, B, n_all, row_offset, S, inv_gb, m->row_loss))) return rc;
+  if ((rc = launch_sampling_loss(m, loss, tanh_out, m->logits, ldc, m->bc, pop, B, n_all, row_offset, S, inv_gb, m->row_loss))) return rc;
   if ((rc = launch_reduce_cost(m, m->row_loss, B, m->grads + m->cost_slot))) return rc;
   if ((rc = launch_gemm(m, true, false, nc, H, B, m->logits, ldc, m->h_last, H, m->dWc, H, 1.f, 0.f))) return rc;
   CU_TRY(m, cudaMemsetAsync(bcg, 0, (size_t)nc * sizeof(float), m->stream));
   if ((rc = launch_colsum(m, m->logits, B, nc, ldc, bcg))) return rc;
   if ((rc = launch_scatter_table_rows(m, m->dWc, bcg, m->cells, nc, H, m->grads + m->out_WT, m->grads + m->out_b))) return rc;
-  if ((rc = launch_gemm(m, false, false, B, H, nc, m->logits, ldc, m->Wc, H, m->dh_last, H, 1.f, 0.f))) return rc;
-  stage_mark(m, 4);
-  if ((rc = backward_stack(m, s))) return rc;
-  return finish_step(m, cost);
+  return launch_gemm(m, false, false, B, H, nc, m->logits, ldc, m->Wc, H, m->dh_last, H, 1.f, 0.f);
 }
 
 struct MarginRagged { bool on = false; bool has_default = false; int exclude_seen = 0; int max_special = 0; };
@@ -1224,6 +1299,24 @@ extern "C" int sbr_scores(sbr_model* m, const int32_t* X, const float* mask, int
   return 0;
 }
 
+// ragged exclusion lists -> m->excl_off / m->excl_ids (*d_off stays NULL when there are none)
+static int upload_exclusions(sbr_model* m, int B, const int32_t* excl_offsets, const int32_t* excl_ids, const int32_t** d_off) {
+  int rc;
+  *d_off = nullptr;
+  if (!excl_offsets || !excl_ids) return 0;
+  const int ne = excl_offsets[B];
+  if (ne > m->excl_cap) {
+    if (m->excl_ids) cudaFree(m->excl_ids);
+    m->excl_ids = nullptr;
+    m->excl_cap = std::max(ne, 2 * m->excl_cap);
+    if ((rc = dev_alloc(m, &m->excl_ids, (size_t)m->excl_cap, false))) return rc;
+  }
+  CU_TRY(m, cudaMemcpyAsync(m->excl_off, excl_offsets, (size_t)(B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  if (ne > 0) CU_TRY(m, cudaMemcpyAsync(m->excl_ids, excl_ids, (size_t)ne * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  *d_off = m->excl_off;
+  return 0;
+}
+
 extern "C" int sbr_topk(sbr_model* m, const int32_t* X, const float* mask, int B, const int32_t* excl_offsets,
                         const int32_t* excl_ids, int k, int mode, int32_t* ids_out) {
   CHECK_STICKY(m);
@@ -1232,21 +1325,195 @@ extern "C" int sbr_topk(sbr_model* m, const int32_t* X, const float* mask, int B
   int rc = scores_device(m, X, mask, B, sm);
   if (rc) return rc;
   const int32_t* d_off = nullptr;
-  if (excl_offsets && excl_ids) {
-    const int ne = excl_offsets[B];
-    if (ne > m->excl_cap) {
-      if (m->excl_ids) cudaFree(m->excl_ids);
-      m->excl_ids = nullptr;
-      m->excl_cap = std::max(ne, 2 * m->excl_cap);
-      if ((rc = dev_alloc(m, &m->excl_ids, (size_t)m->excl_cap, false))) return rc;
-    }
-    CU_TRY(m, cudaMemcpyAsync(m->excl_off, excl_offsets, (size_t)(B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
-    if (ne > 0) CU_TRY(m, cudaMemcpyAsync(m->excl_ids, excl_ids, (size_t)ne * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
-    d_off = m->excl_off;
-  }
+  if ((rc = upload_exclusions(m, B, excl_offsets, excl_ids, &d_off))) return rc;
   if ((rc = launch_topk(m, m->logits, (int)round_up(m->N, 4), B, m->N, d_off, m->excl_ids, k, (mode >> 1) & 1, m->topk_ids))) return rc;
   CU_TRY(m, cudaMemcpyAsync(ids_out, m->topk_ids, (size_t)B * k * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
   CU_TRY(m, cudaStreamSynchronize(m->stream));
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// RNNCluster (rnn_cluster.py)
+// ------------------------------------------------------------------------------------------------
+// The cluster branch of one step (rnn_cluster.py:232-251), after the recommendation branch.  It reads h_last but sends
+// no gradient back to it: the cluster cost only reaches Wc and R (rnn_cluster.py:268-270).
+static int cluster_branch(sbr_model* m, int B, int n_all, int row_offset, int Sc, bool noise, float scale, float inv_gb) {
+  int rc;
+  const int C = m->n_clusters, H = m->H_last, nc = n_all + Sc, lds = (int)round_up(nc, 4), type = m->cluster_type;
+  const float* R = m->params + m->cl_R;
+  if ((rc = launch_gemm(m, false, false, B, C, H, m->h_last, H, m->params + m->cl_W, C, m->cq, C, 1.f, 0.f))) return rc;
+  if ((rc = launch_cluster_select(m, m->cq, noise ? m->cnoise : nullptr, B, C, scale, m->cP))) return rc;
+  if ((rc = launch_cluster_members(m, R, m->ccells, nc, C, type, scale, m->cM))) return rc;
+  if ((rc = launch_gemm(m, false, true, B, nc, C, m->cP, C, m->cM, C, m->cS, lds, 1.f, 0.f))) return rc;
+  if ((rc = launch_sampling_loss(m, m->cluster_loss, false, m->cS, lds, nullptr, nullptr, B, n_all, row_offset, Sc, inv_gb, m->crow_loss))) return rc;
+  if ((rc = launch_reduce_cost(m, m->crow_loss, B, m->grads + m->cost_slot + 1))) return rc;
+  // dP = dS M, dM = dS^T P
+  if ((rc = launch_gemm(m, false, false, B, C, nc, m->cS, lds, m->cM, C, m->cdP, C, 1.f, 0.f))) return rc;
+  if ((rc = launch_gemm(m, true, false, nc, C, B, m->cS, lds, m->cP, C, m->cdM, C, 1.f, 0.f))) return rc;
+  if ((rc = launch_cluster_dq(m, m->cP, m->cdP, B, C, scale, m->cdq))) return rc;
+  if ((rc = launch_gemm(m, true, false, H, C, B, m->h_last, H, m->cdq, C, m->grads + m->cl_W, C, 1.f, 1.f))) return rc;
+  return launch_cluster_dR(m, R, m->ccells, nc, C, type, scale, m->cdM, m->grads + m->cl_R);
+}
+
+extern "C" int sbr_train_step_cluster(sbr_model* m, const int32_t* X, const float* mask, const int32_t* Y_all, int n_all,
+                                      int row_offset, const int32_t* samples, int S, const int32_t* cluster_samples, int Sc,
+                                      const float* noise, float scale, int B, float* cost, float* cluster_cost) {
+  CHECK_STICKY(m);
+  if (m->n_clusters <= 0) { sbr_set_error(m, SBR_E_ARG, "model was not created with sbr_create_cluster"); return SBR_E_ARG; }
+  if (!cluster_samples) Sc = S;
+  if (!Y_all || !samples || S < 1 || S > m->cfg.n_samples || Sc < 1 || Sc > m->n_csamples || n_all < B || n_all > m->global_batch ||
+      row_offset < 0 || row_offset + B > n_all || !(scale == scale)) {
+    sbr_set_error(m, SBR_E_ARG, "bad cluster-step arguments (S=%d Sc=%d n_all=%d row_offset=%d B=%d)", S, Sc, n_all, row_offset, B);
+    return SBR_E_ARG;
+  }
+  const int32_t* cs = cluster_samples ? cluster_samples : samples;
+  int rc;
+  if ((rc = begin_step(m))) return rc;
+  stage_mark(m, 0);
+  BatchSlot& s = m->slots[0];
+  if ((rc = stage_common(m, s, X, mask, B))) return rc;
+  for (int i = 0; i < n_all + std::max(S, Sc); ++i) {
+    const int a = i < n_all ? Y_all[i] : (i - n_all < S ? samples[i - n_all] : 0);
+    const int b = i < n_all ? 0 : (i - n_all < Sc ? cs[i - n_all] : 0);
+    if (a < 0 || a >= m->N || b < 0 || b >= m->N) { sbr_set_error(m, SBR_E_RANGE, "target/sample id outside [0,%d)", m->N); return SBR_E_RANGE; }
+  }
+  CU_TRY(m, cudaMemcpyAsync(m->cells, Y_all, (size_t)n_all * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  CU_TRY(m, cudaMemcpyAsync(m->cells + n_all, samples, (size_t)S * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  CU_TRY(m, cudaMemcpyAsync(m->ccells, Y_all, (size_t)n_all * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  CU_TRY(m, cudaMemcpyAsync(m->ccells + n_all, cs, (size_t)Sc * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  if (noise) CU_TRY(m, cudaMemcpyAsync(m->cnoise, noise, (size_t)B * m->n_clusters * sizeof(float), cudaMemcpyHostToDevice, m->stream));
+  CU_TRY(m, cudaStreamSynchronize(m->stream));
+  const float inv_gb = 1.f / (float)(m->cfg.global_batch > 0 ? m->cfg.global_batch : s.B * m->cfg.n_ranks);
+  if ((rc = forward_stack(m, s))) return rc;
+  // recommendation branch: the sampled model's BlackoutLayer with unit weights and no tanh (rnn_cluster.py:222-228)
+  if ((rc = sampled_output(m, m->cluster_loss, false, nullptr, B, n_all, row_offset, S, inv_gb))) return rc;
+  if ((rc = cluster_branch(m, B, n_all, row_offset, Sc, noise != nullptr, scale, inv_gb))) return rc;
+  stage_mark(m, 4);
+  if ((rc = backward_stack(m, s))) return rc;
+  float local_cost;
+  if ((rc = finish_step(m, cost ? cost : &local_cost))) return rc;
+  if (cluster_cost) *cluster_cost = m->h_cost[1];
+  return 0;
+}
+
+extern "C" int sbr_cluster_test_topk(sbr_model* m, const int32_t* X, const float* mask, int B, const int32_t* excl_offsets,
+                                     const int32_t* excl_ids, int k, int32_t* ids_full, int32_t* ids_cluster,
+                                     int32_t* selected, float* n_used) {
+  CHECK_STICKY(m);
+  if (m->n_clusters <= 0) { sbr_set_error(m, SBR_E_ARG, "model was not created with sbr_create_cluster"); return SBR_E_ARG; }
+  if (!ids_full || !ids_cluster || !selected || !n_used || k < 1 || k > 64 || k > m->N) {
+    sbr_set_error(m, SBR_E_ARG, "cluster_test_topk: bad arguments (k must be in [1, min(64, n_items)])");
+    return SBR_E_ARG;
+  }
+  int rc = scores_device(m, X, mask, B, /*softmax=*/1);
+  if (rc) return rc;
+  const int N = m->N, C = m->n_clusters, H = m->H_last, ld = (int)round_up(N, 4);
+  if (!m->logits2 && (rc = dev_alloc(m, &m->logits2, (size_t)m->B * ld, false))) return rc;
+  if ((rc = launch_gemm(m, false, false, B, C, H, m->h_last, H, m->params + m->cl_W, C, m->cq, C, 1.f, 0.f))) return rc;
+  if ((rc = launch_cluster_hard(m, m->logits, ld, m->cq, m->params + m->cl_R, B, N, C, m->cluster_type, m->logits2, m->csel, m->cnused))) return rc;
+  const int32_t* d_off = nullptr;
+  if ((rc = upload_exclusions(m, B, excl_offsets, excl_ids, &d_off))) return rc;
+  if ((rc = launch_topk(m, m->logits, ld, B, N, d_off, m->excl_ids, k, 0, m->topk_ids))) return rc;
+  CU_TRY(m, cudaMemcpyAsync(ids_full, m->topk_ids, (size_t)B * k * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
+  if ((rc = launch_topk(m, m->logits2, ld, B, N, d_off, m->excl_ids, k, 0, m->topk_ids))) return rc;
+  CU_TRY(m, cudaMemcpyAsync(ids_cluster, m->topk_ids, (size_t)B * k * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
+  CU_TRY(m, cudaMemcpyAsync(selected, m->csel, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
+  CU_TRY(m, cudaMemcpyAsync(n_used, m->cnused, (size_t)B * sizeof(float), cudaMemcpyDeviceToHost, m->stream));
+  CU_TRY(m, cudaStreamSynchronize(m->stream));
+  return 0;
+}
+
+extern "C" int sbr_cluster_build(sbr_model* m, int32_t* sizes) {
+  CHECK_STICKY(m);
+  if (m->n_clusters <= 0) { sbr_set_error(m, SBR_E_ARG, "model was not created with sbr_create_cluster"); return SBR_E_ARG; }
+  CU_TRY(m, cudaSetDevice(m->dev));
+  const int N = m->N, C = m->n_clusters;
+  int rc;
+  if ((rc = launch_cluster_csr(m, m->params + m->cl_R, N, C))) return rc;
+  std::vector<int32_t> off(C + 1);
+  CU_TRY(m, cudaMemcpyAsync(off.data(), m->cl_off, (C + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
+  CU_TRY(m, cudaStreamSynchronize(m->stream));
+  const int64_t total = off[C];
+  int max_size = 0;
+  for (int j = 0; j < C; ++j) max_size = std::max(max_size, off[j + 1] - off[j]);
+  if (total > m->cl_cap_items || !m->cl_items) {
+    if (m->cl_items) cudaFree(m->cl_items);
+    m->cl_items = nullptr;
+    m->cl_cap_items = std::max<int64_t>(total, 1);
+    if ((rc = dev_alloc(m, &m->cl_items, (size_t)m->cl_cap_items, false))) return rc;
+  }
+  if (max_size > m->cl_cap_rows || !m->cl_Wg) {
+    if (m->cl_Wg) cudaFree(m->cl_Wg);
+    m->cl_Wg = nullptr;
+    m->cl_cap_rows = std::max(max_size, 1);
+    if ((rc = dev_alloc(m, &m->cl_Wg, (size_t)m->cl_cap_rows * m->H_last, false))) return rc;
+  }
+  if ((rc = launch_cluster_fill(m, m->params + m->cl_R, N, C))) return rc;
+  CU_TRY(m, cudaStreamSynchronize(m->stream));
+  m->cl_hoff = off;
+  if (sizes)
+    for (int j = 0; j < C; ++j) sizes[j] = off[j + 1] - off[j];
+  return 0;
+}
+
+extern "C" int sbr_cluster_topk(sbr_model* m, const int32_t* X, const float* mask, int B, const int32_t* excl_offsets,
+                                const int32_t* excl_ids, int k, int32_t* ids_out, int32_t* n_out, int32_t* selected_out,
+                                int use_clusters) {
+  CHECK_STICKY(m);
+  if (m->n_clusters <= 0) { sbr_set_error(m, SBR_E_ARG, "model was not created with sbr_create_cluster"); return SBR_E_ARG; }
+  if (!ids_out || !n_out || k < 1 || k > 64 || k > m->N) { sbr_set_error(m, SBR_E_ARG, "cluster_topk: k must be in [1, min(64, n_items)]"); return SBR_E_ARG; }
+  const int N = m->N, C = m->n_clusters, H = m->H_last;
+  int rc;
+  if (!use_clusters) {   // --ignore_clusters: the whole catalog, raw scores, -inf exclusion (rnn_cluster.py:314-321)
+    if ((rc = sbr_topk(m, X, mask, B, excl_offsets, excl_ids, k, 2, ids_out))) return rc;
+    for (int b = 0; b < B; ++b) n_out[b] = N;
+    if (selected_out)
+      for (int b = 0; b < B; ++b) selected_out[b] = -1;
+    return 0;
+  }
+  if (m->cl_hoff.empty()) { sbr_set_error(m, SBR_E_ARG, "cluster_topk: call sbr_cluster_build first"); return SBR_E_ARG; }
+  BatchSlot& s = m->slots[0];
+  CU_TRY(m, cudaSetDevice(m->dev));
+  if ((rc = stage_common(m, s, X, mask, B))) return rc;
+  const bool prof = m->profiling;
+  m->profiling = false;
+  rc = forward_stack(m, s);
+  m->profiling = prof;
+  if (rc) return rc;
+  if ((rc = launch_gemm(m, false, false, B, C, H, m->h_last, H, m->params + m->cl_W, C, m->cq, C, 1.f, 0.f))) return rc;
+  if ((rc = launch_cluster_argmax(m, m->cq, B, C, m->csel))) return rc;
+  std::vector<int32_t> sel(B), perm(B);
+  CU_TRY(m, cudaMemcpyAsync(sel.data(), m->csel, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
+  CU_TRY(m, cudaStreamSynchronize(m->stream));
+  // rows grouped by selected cluster: each cluster's item rows are gathered once and scored by one GEMM
+  for (int b = 0; b < B; ++b) perm[b] = b;
+  std::stable_sort(perm.begin(), perm.end(), [&](int a, int b) { return sel[a] < sel[b]; });
+  const std::vector<int32_t>& off = m->cl_hoff;
+  int ld = 4;
+  for (int b = 0; b < B; ++b) ld = std::max<int>(ld, (int)round_up(off[sel[b] + 1] - off[sel[b]], 4));
+  CU_TRY(m, cudaMemcpyAsync(m->cperm, perm.data(), (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, m->stream));
+  if ((rc = launch_gather_table_rows(m, m->h_last, nullptr, m->cperm, B, H, m->ch_sorted, nullptr))) return rc;
+  for (int r0 = 0; r0 < B;) {
+    const int c = sel[perm[r0]];
+    int r1 = r0;
+    while (r1 < B && sel[perm[r1]] == c) ++r1;
+    const int nc = off[c + 1] - off[c];
+    if (nc > 0) {
+      if ((rc = launch_gather_table_rows(m, m->params + m->out_WT, nullptr, m->cl_items + off[c], nc, H, m->cl_Wg, nullptr))) return rc;
+      if ((rc = launch_gemm(m, false, true, r1 - r0, nc, H, m->ch_sorted + (size_t)r0 * H, H, m->cl_Wg, H, m->logits + (size_t)r0 * ld, ld,
+                            1.f, 0.f))) return rc;
+    }
+    r0 = r1;
+  }
+  const int32_t* d_off = nullptr;
+  if ((rc = upload_exclusions(m, B, excl_offsets, excl_ids, &d_off))) return rc;
+  if ((rc = launch_cluster_row_topk(m, m->logits, ld, B, m->cperm, m->csel, m->params + m->out_b, d_off, m->excl_ids, k, m->topk_ids))) return rc;
+  CU_TRY(m, cudaMemcpyAsync(ids_out, m->topk_ids, (size_t)B * k * sizeof(int32_t), cudaMemcpyDeviceToHost, m->stream));
+  CU_TRY(m, cudaStreamSynchronize(m->stream));
+  for (int b = 0; b < B; ++b) {
+    n_out[b] = off[sel[b] + 1] - off[sel[b]];
+    if (selected_out) selected_out[b] = sel[b];
+  }
   return 0;
 }
 

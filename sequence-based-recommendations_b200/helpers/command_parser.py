@@ -1,10 +1,11 @@
 """Command-line flags and the predictor factory -- host mirror of helpers/command_parser.py:22-127
 restricted to the RNN method (the path this build accelerates).  Every flag of the reference's
-parser is kept so existing command lines still parse; methods other than ``-m RNN`` and the
-clustered RNN (``--clusters``) raise NotImplementedError (SURVEY.md §2 rows 9-10, 16-19)."""
+parser is kept so existing command lines still parse; methods other than ``-m RNN`` raise NotImplementedError
+(SURVEY.md §2 rows 9-10, 16-19).  ``-m RNN --clusters K`` builds the clustered RNN (command_parser.py:114-115)."""
 import argparse
 
 from ..neural_networks.recurrent_layers import get_recurrent_layers, recurrent_layers_command_parser
+from ..neural_networks.rnn_cluster import RNNCluster
 from ..neural_networks.rnn_margin import RNNMargin
 from ..neural_networks.rnn_one_hot import RNNOneHot
 from ..neural_networks.rnn_sampling import RNNSampling
@@ -92,14 +93,17 @@ def get_predictor(args, **dist):
     data-parallel placement (device, n_ranks, rank, nccl_id)."""
     if args.method != 'RNN':
         raise NotImplementedError("-m %s: only the RNN method is on the B200 hot path (SURVEY.md §8)" % args.method)
-    if args.clusters > 0:
-        raise NotImplementedError("--clusters (RNNCluster) is outside the B200 hot path (SURVEY.md §2 row 9)")
     common = dict(interactions_are_unique=(not args.repeated_interactions), max_length=args.max_length,
                   updater=get_update_manager(args), target_selection=get_target_selection(args),
                   sequence_noise=get_sequence_noise(args), recurrent_layer=get_recurrent_layers(args),
                   use_ratings_features=args.rf, use_movies_features=args.mf, use_users_features=args.uf,
                   batch_size=args.batch_size, prefetch_batches=getattr(args, 'prefetch', 0))
     common.update(dist)
+    if args.clusters > 0:       # checked before the loss dispatch, as in the reference
+        return RNNCluster(cluster_selection_noise=args.csn, loss=args.loss, predict_with_clusters=(not args.ignore_clusters),
+                          sampling_bias=args.sampling_bias, sampling=args.sampling, cluster_sampling=args.c_sampling,
+                          init_scale=args.init_scale, scale_growing_rate=args.scale_growing_rate,
+                          max_scale=args.max_scale, n_clusters=args.clusters, cluster_type=args.cluster_type, **common)
     if args.loss == 'CCE':
         return RNNOneHot(diversity_bias=args.diversity_bias, regularization=args.regularization, **common)
     if args.loss in ('hinge', 'logit', 'logsig'):

@@ -186,28 +186,31 @@ class RNNBase(object):
         sparse_lstm.py:156-159,590-593,960-961); learned cell_init / hid_init = 0; EmbeddingLayer.W ~ Normal(std
         0.01) (recurrent_layers.py:47); Dense / Blackout W ~ GlorotUniform(gain) (rnn_one_hot.py:65,
         rnn_sampling.py:131, rnn_margin.py:103), b = 0."""
-        if self.init_seed is None:
-            rng = np.random.RandomState(20160901) if self.n_ranks > 1 else np.random
-        else:
-            rng = np.random.RandomState(self.init_seed)
-        vals = []
-        for name, shape in self.engine.param_infos():
-            leaf = name.split(".")[1]
-            if name == "emb.W":
-                v = rng.normal(0.0, 0.01, size=shape)
-            elif name == "out.W":
-                a = float(self.last_layer_init) * np.sqrt(6.0 / (shape[0] + shape[1]))
-                v = rng.uniform(-a, a, size=shape)
-            elif leaf in ("W_in_to_hid", "W_hid_to_hid"):
-                # Vanilla layers with a dense input are lasagne.layers.RecurrentLayer (recurrent_layers.py:98-99),
-                # whose weights default to lasagne.init.Uniform() = U(-0.01, 0.01)
-                v = rng.uniform(-0.01, 0.01, size=shape)
-            elif leaf.startswith("W_"):
-                v = rng.normal(0.0, 0.1, size=shape)
-            else:
-                v = np.zeros(shape, dtype=np.float32)
-            vals.append(np.asarray(v, dtype=np.float32))     # drawn in float64 like Lasagne, stored as floatX
+        rng = self._init_rng()
+        vals = [self._initial_value(rng, name, shape) for name, shape in self.engine.param_infos()]
         self.engine.set_all_param_values(vals)
+
+    def _init_rng(self):
+        if self.init_seed is None:
+            return np.random.RandomState(20160901) if self.n_ranks > 1 else np.random
+        return np.random.RandomState(self.init_seed)
+
+    def _initial_value(self, rng, name, shape):
+        leaf = name.split(".")[1]
+        if name == "emb.W":
+            v = rng.normal(0.0, 0.01, size=shape)
+        elif name == "out.W":
+            a = float(self.last_layer_init) * np.sqrt(6.0 / (shape[0] + shape[1]))
+            v = rng.uniform(-a, a, size=shape)
+        elif leaf in ("W_in_to_hid", "W_hid_to_hid"):
+            # Vanilla layers with a dense input are lasagne.layers.RecurrentLayer (recurrent_layers.py:98-99),
+            # whose weights default to lasagne.init.Uniform() = U(-0.01, 0.01)
+            v = rng.uniform(-0.01, 0.01, size=shape)
+        elif leaf.startswith("W_"):
+            v = rng.normal(0.0, 0.1, size=shape)
+        else:
+            v = np.zeros(shape, dtype=np.float32)
+        return np.asarray(v, dtype=np.float32)     # drawn in float64 like Lasagne, stored as floatX
 
     def _common_filename(self, epochs):
         """Common part of the checkpoint filename across sub classes (rnn_base.py:111-130)."""

@@ -43,15 +43,21 @@ def run_tests(predictor, model_file, dataset, args, get_full_recommendation_list
     if get_full_recommendation_list:
         k = min(dataset.n_items, 64)
     start = time.process_time()
+    nb_of_dp = []
     for sequence, user_id in dataset.test_set(epochs=1):
         num_viewed = int(len(sequence) / 2)
         viewed = sequence[:num_viewed]
         goal = [int(i[0]) for i in sequence[num_viewed:]]
         if len(goal) == 0:
             raise ValueError
-        evaluator.add_instance(goal, predictor.top_k_recommendations(viewed, user_id=user_id, k=k))
+        if getattr(args, 'clusters', -1) > 0:     # the clustered RNN also returns how many items it scored (test.py:61-63)
+            recommendations, n = predictor.top_k_recommendations(viewed, user_id=user_id, k=k)
+            nb_of_dp.append(n)
+        else:
+            recommendations = predictor.top_k_recommendations(viewed, user_id=user_id, k=k)
+        evaluator.add_instance(goal, recommendations)
     print('Timer: ', time.process_time() - start)
-    evaluator.nb_of_dp = dataset.n_items
+    evaluator.nb_of_dp = np.mean(nb_of_dp) if nb_of_dp else dataset.n_items
     return evaluator
 
 
